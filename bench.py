@@ -59,6 +59,17 @@ def synth(seed, B, T, D1, D2, ragged=False):
     return x1, x2, lengths
 
 
+def dump_outputs(out_dir, scores, tags):
+    """What the last timed headline step returned, as <out_dir>/<name>.npy in float32: the head's scores [B, T, n_out]
+    and the thresholded boundary tags [B, T] (255 beyond an episode's length), the batches of all ranks in rank order.
+    The inputs and weights are seeded, so the files of two builds can be compared array for array."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("scores", scores), ("tags", tags)):
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 class ClockSampler:
     """nvidia-smi clocks / throttle reasons sampled DURING the timed region (B200_PROFILING.md recipe)."""
 
@@ -855,8 +866,7 @@ def run_ours(args, rank, world, local_rank):
         x1, x2, lens = dev_sets[i % n_sets]
         with torch.no_grad():
             feats = model.model((x1, x2), lens)
-            scores, tags = ops.head_decode(feats, model.classification.weight, model.classification.bias, lens, 0.5)
-        return tags
+            return ops.head_decode(feats, model.classification.weight, model.classification.bias, lens, 0.5)
 
     def host_batches(n):  # what a DataLoader(pin_memory=True) over the collater yields
         for i in range(n):
@@ -915,15 +925,20 @@ def run_ours(args, rank, world, local_rank):
     clk = ClockSampler(local_rank)   # re-entered around every GPU-busy timed leg; the samples accumulate
     clk.__enter__()
     start.record()
-    tags = None
+    scores = tags = None
     for i in range(args.steps):
-        tags = device_step(i)
+        scores, tags = device_step(i)
     if world > 1:  # inference needs only a final gather of the boundary predictions: once, after the last step
         gathered = mdist.gather_tags(tags)
     end.record()
     barrier()
     launches = ops.launch_count() if graphs is None else launches_per_step * args.steps
     ms = ctx.max_over_ranks(start.elapsed_time(end))
+    if args.dump_outputs:
+        if world > 1:   # every rank takes part in the gather, outside the timed region
+            scores, tags = torch.cat(mdist.gather_tags(scores)), torch.cat(gathered)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, scores, tags)
 
     # ---- per-kernel CUDA-event pass (roofline of the dominant kernel) ------------------------------------
     prof_lists = ctx.profile(eager, n=args.steps)
@@ -1085,7 +1100,13 @@ def main():
                                                    "(the headline leg always runs); 'none' = headline only")
     ap.add_argument("--skip-transformer", action="store_true", help="skip the configs[2] windowed-attention leg")
     ap.add_argument("--no-graph", action="store_true", help="time eager launches instead of CUDA-graph replays")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the scores and tags of the last timed headline step to "
+                                                           "DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA arm (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

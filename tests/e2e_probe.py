@@ -1,5 +1,5 @@
-import sys, time, torch
-sys.path.insert(0, '/root/repo')
+import os, sys, time, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import multimodaltopicsegmentation_b200 as m
 import bench
 dev = torch.device('cuda:0')

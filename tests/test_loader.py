@@ -1,6 +1,6 @@
 """Loader mirror (multimodaltopicsegmentation_b200/load_datasets_precomputed.py) against outputs of the unmodified
-reference loader (tests/golden/loader_split.npz, made by tests/golden/make_golden_loader.py) and, when /root/reference
-is present (build container only), against the reference itself in k-fold mode."""
+reference loader (tests/golden/loader_split.npz, made by tests/golden/make_golden_loader.py) and, in k-fold and
+sentence-masking mode, against the reference itself where it is present and against tests/golden/loader_kfold.npz."""
 import json
 import os
 import pickle
@@ -100,6 +100,36 @@ def test_kfold_and_masking_match_reference_live(golden, tmp_path):
                 assert [e[2] for e in pa] == [e[2] for e in pb]
                 for ea, eb in zip(pa, pb):
                     assert torch.equal(ea[0], eb[0]) and list(ea[1]) == list(eb[1])
+
+
+def test_kfold_and_masking_match_golden(golden, tmp_path, monkeypatch):
+    """k-fold and sentence-masking modes against tests/golden/loader_kfold.npz (made by
+    tests/golden/make_golden_loader_kfold.py), with the directory listing sorted as it was when the file was written.
+    Its `source` entry names the loader that wrote it: this package's, as a regression pin, until it is re-recorded
+    from a reference checkout."""
+    from multimodaltopicsegmentation_b200 import load_dataset_from_precomputed
+
+    fx = golden("loader_kfold")
+    root = str(tmp_path)
+    _rebuild(golden("loader_split"), root)
+    listdir = os.listdir
+    monkeypatch.setattr(os, "listdir", lambda p: sorted(listdir(p)))
+    emb = os.path.join(root, "text") + "+" + os.path.join(root, "audio")
+    lab = os.path.join(root, "labs_dict.pkl")
+    tags = sorted({k.split(":")[0] for k in fx.files if k.endswith(":kwargs")})
+    assert tags == ["kfold2_masked", "kfold3"]
+    for tag in tags:
+        folds = load_dataset_from_precomputed(emb, lab, **json.loads(str(fx[f"{tag}:kwargs"])))
+        assert len(folds) == int(fx[f"{tag}:folds"])
+        for i, fold in enumerate(folds):
+            assert len(fold) == 2
+            for part, eps in zip(("train", "test"), fold):
+                assert [e[2] for e in eps] == fx[f"{tag}:{i}:{part}:names"].tolist()
+                for e in eps:
+                    x = fx[f"{tag}:{i}:{part}:{e[2]}:x"]
+                    assert e[0].numpy().dtype == x.dtype
+                    np.testing.assert_array_equal(e[0].numpy(), x)
+                    assert list(e[1]) == fx[f"{tag}:{i}:{part}:{e[2]}:y"].tolist()
 
 
 @pytest.mark.gpu
