@@ -178,6 +178,30 @@ int mts_gemm_bf16p(const float *A_lo, const float *B_lo, const float *bias, floa
                    int epilogue, int accumulate, void *stream);
 int mts_pack_rows_bf16in(const void *src1, int64_t bstride1, int D1, const void *src2, int64_t bstride2, int D2, int B, int T,
                          int Kp, float *lo, void *stream);
+/* bf16 path of the windowed-attention encoder (inference; replaces, per layer, what HF LongformerLayer computes,
+ * modeling_longformer.py:401-442, 481-639, 1060-1171, from models/RestrictedTransformerLayer.py:131):
+ *   mts_gemm_bf16p_out16     : the q/k/v projection (LongformerSelfAttention.query/key/value, :503-505): mts_gemm_bf16p with
+ *                              the bias epilogue, C stored as bf16 [M, ldc] = round-to-nearest-even of mts_gemm_bf16p's fp32
+ *                              output.  N % 4 == 0, ldc % 4 == 0, Kp <= 3072 (no K split).
+ *   mts_gemm_bf16p_gelu_pair : LongformerIntermediate (:1103-1116): the bf16-product twin of mts_gemm_tf32x3_gelu_pair,
+ *                              C = gelu(A B^T + bias) fp32 [M, N] and its packed operand C_lo [M, N] (side 0).
+ *   mts_embed_ln_fwd_bf16in  : LongformerEmbeddings (:401-442) = mts_embed_ln_fwd reading bf16 embeddings x; writes y fp32 and
+ *                              its packed operand y_lo [rows, Kp] (Kp == d).
+ *   mts_band_attn_fwd_bf16   : LongformerSelfAttention's banded softmax (:481-639, sliding chunks :758-867) over bf16 qkv
+ *                              [rows, ld] (rows = [q | k | v], q not yet scaled; ld % 8 == 0; `rows` = the buffer's row count):
+ *                              S = Q K^T and O += P V as kind::f16 tcgen05.mma with fp32 accumulation, fp32 softmax, P rounded
+ *                              to bf16.  Same masks and padded-query zeros as mts_band_attn_fwd; S <= 4094.  Outputs: out fp32
+ *                              [rows, nheads*hd] and / or out_lo [rows, Kp] (the packed operand of mts_gemm_bf16p, Kp ==
+ *                              nheads*hd); lse [B, nheads, S] or NULL.  Head dims 16, 32, 64, 112, 128 (else MTS_E_UNSUPPORTED). */
+int mts_gemm_bf16p_out16(const float *A_lo, const float *B_lo, const float *bias, void *C, int M, int N, int Kp, int64_t ldc,
+                         void *stream);
+int mts_gemm_bf16p_gelu_pair(const float *A_lo, const float *B_lo, const float *bias, float *C, float *C_lo, int M, int N, int Kp,
+                             void *stream);
+int mts_embed_ln_fwd_bf16in(const void *x, int64_t x_bstride, const float *pos, const float *typ, const float *gamma,
+                            const float *beta, int B, int S, int d, float eps, float *y, float *y_lo, int Kp,
+                            const int32_t *lengths, const int32_t *offsets, void *stream);
+int mts_band_attn_fwd_bf16(const void *qkv, int64_t ld, int64_t rows, const int32_t *lengths, const int32_t *offsets, int B,
+                           int S, int nheads, int hd, int w, float *out, float *out_lo, int Kp, float *lse, void *stream);
 
 /* Profiling hook of the tensor-core recurrence: installs (or, with NULL, removes) a device buffer of 4 x 12 int64
  * into which CTA 0 writes clock64() stamps of the phases of steps 8..11 (see csrc/lstm_rec_tc.cu). */

@@ -41,6 +41,10 @@ SIGNATURES = {
     "mts_gemm_f16x3": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int64, c_int, _P]),
     "mts_gemm_tf32x3_gelu_pair": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int, c_int, c_int, _P]),
     "mts_gemm_bf16p": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int64, c_int, c_int, _P]),
+    "mts_gemm_bf16p_out16": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int64, _P]),
+    "mts_gemm_bf16p_gelu_pair": (c_int, [_P, _P, _P, _P, _P, c_int, c_int, c_int, _P]),
+    "mts_embed_ln_fwd_bf16in": (c_int, [_P, c_int64, _P, _P, _P, _P, c_int, c_int, c_int, c_float, _P, _P, c_int, _P, _P, _P]),
+    "mts_band_attn_fwd_bf16": (c_int, [_P, c_int64, c_int64, _P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P, c_int, _P, _P]),
     "mts_pack_rows_bf16in": (c_int, [_P, c_int64, c_int, _P, c_int64, c_int, c_int, c_int, c_int, _P, _P]),
     "mts_debug_rec_profile": (c_int, [_P]),
     "mts_debug_rec_profile_h3": (c_int, [_P]),

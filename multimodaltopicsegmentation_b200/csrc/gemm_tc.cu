@@ -283,6 +283,33 @@ __device__ __forceinline__ void tc_store_tile(uint32_t tmem_base, int acc_col, i
     }
     return;
   }
+  // epilogue 3 (bf16 precision switch): bias, then C stored as bf16 (round to nearest even; C points to bf16 [M, ldc]) --
+  // the q/k/v projection whose output the bf16 attention kernel reads
+  if (epilogue == 3) {
+    uint16_t *Cb = reinterpret_cast<uint16_t *>(C);
+#pragma unroll 1
+    for (int c0 = 0; c0 < BN; c0 += 32) {
+      if (n0 + c0 >= N) break;
+      const int n = n0 + c0 + 4 * ch;
+      float v[32];
+      tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc_col + c0), v);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) stg[lane * 8 + (j ^ (lane & 7))] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
+      __syncwarp();
+      const bool col_ok = n < N;
+      float4 bv = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (col_ok) bv = make_float4(__ldg(bias + n), __ldg(bias + n + 1), __ldg(bias + n + 2), __ldg(bias + n + 3));
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        const int row = 4 * i + rsub, m = m0 + q * 32 + row;
+        const float4 t = stg[row * 8 + (ch ^ (row & 7))];
+        if (m < M && col_ok)
+          *reinterpret_cast<uint2 *>(Cb + (int64_t)m * ldc + n) = make_uint2(bf16x2_bits(t.x + bv.x, t.y + bv.y), bf16x2_bits(t.z + bv.z, t.w + bv.w));
+      }
+      __syncwarp();
+    }
+    return;
+  }
 #pragma unroll 1
   for (int c0 = 0; c0 < BN; c0 += 32) {
     if (n0 + c0 >= N) break;
@@ -857,7 +884,7 @@ static int launch_tc(const float *A_hi, const float *A_lo, const float *B_hi, co
   // summed with round-to-nearest atomics keep the product inside the 2e-5 contract at any K.
   int splits = 1;
   const int num_kb = Kp / TC_BK;
-  if (epilogue != 2 && !C_lo) {
+  if (epilogue < 2 && !C_lo) {   // (epilogue 2: GELU, 3: bf16 output -- neither can be summed over K splits)
     if (tiles * 2 <= slots && num_kb >= 32) {
       splits = slots / tiles;
       if (splits > num_kb / 8) splits = num_kb / 8;
@@ -998,4 +1025,34 @@ extern "C" int mts_gemm_bf16p(const float *A_lo, const float *B_lo, const float 
   cudaStream_t st = (cudaStream_t)stream;
   if (N >= 256) return launch_tc<256>(A_lo, A_lo, B_lo, B_lo, bias, C, M, N, Kp, ldc, epilogue, accumulate, st, 1);
   return launch_tc<128>(A_lo, A_lo, B_lo, B_lo, bias, C, M, N, Kp, ldc, epilogue, accumulate, st, 1);
+}
+
+// mts_gemm_bf16p with epilogue 3: C = bf16(A B^T + bias), stored as bf16 [M, ldc] (round to nearest even of the fp32 value
+// mts_gemm_bf16p's bias epilogue writes).  Feeds mts_band_attn_fwd_bf16 (the q/k/v projection, C = qkv).  No K split:
+// Kp <= 3072 (the bound the fused-activation forms keep too).
+extern "C" int mts_gemm_bf16p_out16(const float *A_lo, const float *B_lo, const float *bias, void *C, int M, int N, int Kp,
+                                    int64_t ldc, void *stream) {
+  MTS_REQUIRE(A_lo && B_lo && bias && C, MTS_E_BADARG, "gemm_bf16p_out16: null pointer");
+  MTS_REQUIRE(M > 0 && N > 0 && Kp > 0, MTS_E_BADARG, "gemm_bf16p_out16: empty shape");
+  MTS_REQUIRE(Kp % TC_BK == 0 && Kp <= 3072, MTS_E_UNSUPPORTED, "gemm_bf16p_out16: Kp must be a multiple of 32 and <= 3072");
+  MTS_REQUIRE(N % 4 == 0 && ldc % 4 == 0 && ldc >= N, MTS_E_UNSUPPORTED, "gemm_bf16p_out16: N and ldc must be multiples of 4, ldc >= N");
+  MTS_REQUIRE((((uintptr_t)A_lo | (uintptr_t)B_lo | (uintptr_t)C) & 15) == 0, MTS_E_BADARG, "gemm_bf16p_out16: operands must be 16-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (N >= 256) return launch_tc<256>(A_lo, A_lo, B_lo, B_lo, bias, (float *)C, M, N, Kp, ldc, 3, 0, st, 1);
+  return launch_tc<128>(A_lo, A_lo, B_lo, B_lo, bias, (float *)C, M, N, Kp, ldc, 3, 0, st, 1);
+}
+
+// The bf16-product twin of mts_gemm_tf32x3_gelu_pair: C = gelu(A B^T + bias) fp32 [M, N] and C_lo [M, N] = its packed operand
+// (side 0), from the packed operands alone (A_lo, B_lo as mts_gemm_bf16p reads them).  N % 32 == 0, ldc == N, Kp <= 3072.
+extern "C" int mts_gemm_bf16p_gelu_pair(const float *A_lo, const float *B_lo, const float *bias, float *C, float *C_lo, int M, int N,
+                                        int Kp, void *stream) {
+  MTS_REQUIRE(A_lo && B_lo && bias && C && C_lo, MTS_E_BADARG, "gemm_bf16p_gelu_pair: null pointer");
+  MTS_REQUIRE(M > 0 && N > 0 && Kp > 0, MTS_E_BADARG, "gemm_bf16p_gelu_pair: empty shape");
+  MTS_REQUIRE(Kp % TC_BK == 0 && N % 32 == 0, MTS_E_UNSUPPORTED, "gemm_bf16p_gelu_pair: Kp and N must be multiples of 32");
+  MTS_REQUIRE(Kp <= 3072, MTS_E_UNSUPPORTED, "gemm_bf16p_gelu_pair: K beyond 3072 needs the split-K path (no fused activation)");
+  MTS_REQUIRE((((uintptr_t)A_lo | (uintptr_t)B_lo | (uintptr_t)C | (uintptr_t)C_lo) & 15) == 0, MTS_E_BADARG,
+              "gemm_bf16p_gelu_pair: operands must be 16-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (N >= 256) return launch_tc<256>(A_lo, A_lo, B_lo, B_lo, bias, C, M, N, Kp, N, 2, 0, st, 1, C_lo);
+  return launch_tc<128>(A_lo, A_lo, B_lo, B_lo, bias, C, M, N, Kp, N, 2, 0, st, 1, C_lo);
 }

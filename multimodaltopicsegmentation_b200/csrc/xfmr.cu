@@ -24,6 +24,7 @@ namespace mts {
 // LayerNorm forward, one warp per token row, values held in registers (two-pass mean / variance).
 //   MODE 0: v = x[b, t, :] + pos[t + 2, :] + typ[:]       (embeddings; position ids start at pad_token_id + 1 = 2)
 //   MODE 1: v = a[row, :] + res[row, :]                    (dense output + residual)
+//   MODE 2: MODE 0 with x given as bf16                    (embeddings stored and shipped in bf16: half the host-to-device bytes)
 // outputs: y fp32, optional (hi, lo) TF32 halves [M, Kp] for the next GEMM, optional pre-LN sum and
 // (mean, rstd) for the backward pass.
 // ---------------------------------------------------------------------------------------------------------
@@ -47,13 +48,16 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const float *__restrict__ a
   for (int in_row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; in_row < M; in_row += warps) {
     const float4 *pa, *pb;
     int row = in_row;
-    if (MODE == 0) {
+    if (MODE != 1) {
       const int bi = in_row / S, t = in_row % S;
       if (offsets) {  // ragged output: valid sentences only, episode bi starts at row offsets[bi]
         if (t >= lengths[bi]) continue;
         row = offsets[bi] + t;
       }
-      pa = reinterpret_cast<const float4 *>(a + (int64_t)bi * a_bstride + (int64_t)t * d);
+      if (MODE == 2)   // 4 bf16 (8 bytes) per float4 column: pa is only a row address here, read as uint2 below
+        pa = reinterpret_cast<const float4 *>(reinterpret_cast<const uint16_t *>(a) + (int64_t)bi * a_bstride + (int64_t)t * d);
+      else
+        pa = reinterpret_cast<const float4 *>(a + (int64_t)bi * a_bstride + (int64_t)t * d);
       pb = reinterpret_cast<const float4 *>(b + (int64_t)(t + 2) * d);
     } else {
       pa = reinterpret_cast<const float4 *>(a + (int64_t)row * d);
@@ -68,12 +72,19 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const float *__restrict__ a
     for (int i = 0; i < MAXV; ++i) {
       const int c = LN_COL(i);
       if (c < nv) {
-        float4 x = __ldg(pa + c);
-        if (MODE == 0 || pb) {
+        float4 x;
+        if (MODE == 2) {
+          const uint2 u = __ldg(reinterpret_cast<const uint2 *>(pa) + c);
+          x = make_float4(__uint_as_float(u.x << 16), __uint_as_float(u.x & 0xFFFF0000u), __uint_as_float(u.y << 16),
+                          __uint_as_float(u.y & 0xFFFF0000u));
+        } else {
+          x = __ldg(pa + c);
+        }
+        if (MODE != 1 || pb) {
           const float4 r = __ldg(pb + c);
           x.x += r.x; x.y += r.y; x.z += r.z; x.w += r.w;
         }
-        if (MODE == 0) {
+        if (MODE != 1) {
           const float4 e = __ldg(reinterpret_cast<const float4 *>(typ) + c);
           x.x += e.x; x.y += e.y; x.z += e.z; x.w += e.w;
         }
@@ -729,6 +740,30 @@ extern "C" int mts_add_ln_fwd(const float *a, const float *res, const float *gam
   else
     ln_fwd_kernel<1, 16><<<grid, 256, 0, (cudaStream_t)stream>>>(a, 0, res, nullptr, gamma, beta, M, 0, d, eps, y, y_hi, y_lo,
                                                                   Kp, sum_out, stats, nullptr, nullptr);
+  MTS_LAUNCH_CHECK();
+  return 0;
+}
+
+// mts_embed_ln_fwd reading bf16 embeddings x (element stride x_bstride between episodes): y fp32 and its packed operand y_lo
+// [rows, Kp] (side 0), the A operand of mts_gemm_bf16p / mts_gemm_bf16p_out16.  Everything after the load is mts_embed_ln_fwd's.
+extern "C" int mts_embed_ln_fwd_bf16in(const void *x, int64_t x_bstride, const float *pos, const float *typ, const float *gamma,
+                                       const float *beta, int B, int S, int d, float eps, float *y, float *y_lo, int Kp,
+                                       const int32_t *lengths, const int32_t *offsets, void *stream) {
+  MTS_REQUIRE(x && pos && typ && gamma && beta && y, MTS_E_BADARG, "embed_ln_fwd_bf16in: null pointer");
+  MTS_REQUIRE(!offsets || lengths, MTS_E_BADARG, "embed_ln_fwd_bf16in: ragged output needs the lengths");
+  MTS_REQUIRE(B > 0 && S > 0, MTS_E_BADARG, "embed_ln_fwd_bf16in: empty shape");
+  MTS_REQUIRE(((uintptr_t)x & 7) == 0 && x_bstride % 4 == 0, MTS_E_BADARG, "embed_ln_fwd_bf16in: x must be 8-byte aligned, stride a multiple of 4");
+  int rc = ln_args_ok("embed_ln_fwd_bf16in", B * S, d, nullptr, y_lo, Kp);
+  if (rc) return rc;
+  const int M = B * S;
+  const float *xf = reinterpret_cast<const float *>(x);
+  const unsigned grid = (unsigned)min((int64_t)(M + 7) / 8, (int64_t)kNumSMs * 8);
+  if (d <= 1024)
+    ln_fwd_kernel<2, 8><<<grid, 256, 0, (cudaStream_t)stream>>>(xf, x_bstride, pos, typ, gamma, beta, M, S, d, eps, y, nullptr, y_lo,
+                                                                 Kp, nullptr, nullptr, lengths, offsets);
+  else
+    ln_fwd_kernel<2, 16><<<grid, 256, 0, (cudaStream_t)stream>>>(xf, x_bstride, pos, typ, gamma, beta, M, S, d, eps, y, nullptr, y_lo,
+                                                                  Kp, nullptr, nullptr, lengths, offsets);
   MTS_LAUNCH_CHECK();
   return 0;
 }

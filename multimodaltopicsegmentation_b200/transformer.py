@@ -171,6 +171,20 @@ class PackedEncoder:
                 ent["w1_p"] = ops.f16_pieces(lyr.intermediate.dense.weight.detach())
         return ent
 
+    def packed_bf16(self, l):
+        """bf16 path: the four dense weights packed like A operands (side 0, mts_split_tf32) so that the packed halves of
+        activations and weights pair up x * w in mts_gemm_bf16p.  Made on first use per weight version, inference only."""
+        ent = self.get()[l]
+        if "wqkv_bf" not in ent:
+            lyr = self.params.encoder.layer[l]
+            sa = lyr.attention.self
+            with torch.no_grad():
+                wqkv = torch.cat([sa.query.weight, sa.key.weight, sa.value.weight], dim=0).contiguous()
+                for name, w in (("wqkv_bf", wqkv), ("wo_bf", lyr.attention.output.dense.weight), ("w1_bf", lyr.intermediate.dense.weight),
+                                ("w2_bf", lyr.output.dense.weight)):
+                    ent[name] = ops.split_tf32(w.detach().contiguous(), side=ops.A_SIDE)[1]
+        return ent
+
     def transposed(self, l):
         """hi/lo of W^T for the dX GEMMs of the backward pass (made on first use per weight version)."""
         ent = self.get()[l]
@@ -353,6 +367,75 @@ def encoder_forward_f16(x, lens, packed: PackedEncoder, nheads, reaches):
     return h.view(B, S, d)
 
 
+def _bf16_eligible(d, nheads):
+    """The bf16 encoder (ops.set_precision("bf16")) serves widths that are whole 32-column blocks (the packed operands carry no K
+    padding) and the head dims of the tcgen05 attention kernels; everything else keeps the fp32 path."""
+    return (ops.PRECISION == "bf16" and _pad32(d) == d and d <= 2048
+            and ops._lib.load().mts_band_attn_tc_supported(d // nheads) != 0)
+
+
+def encoder_forward_bf16(x, lens, packed: PackedEncoder, nheads, reaches):
+    """Inference pass of the encoder under the bf16 precision switch: every dense layer is a bf16 x bf16 product
+    (mts_gemm_bf16p and its epilogue forms) over the packed operands the producers write, q/k/v are bf16 and the banded
+    attention runs on bf16 operands (mts_band_attn_fwd_bf16):
+
+        emb LN (h, h_lo) -> QKV [bf16p_out16, bf16 qkv] -> band_attn_fwd_bf16 -> a_lo -> out-proj [bf16p] -> LN(t + h) (y, y_lo)
+               -> intermediate dense + GELU [bf16p_gelu_pair: z, z_lo] -> output dense [bf16p] -> LN(u + y) -> ...
+
+    The residual stream, the LayerNorm statistics, the softmax, all accumulators and the returned hidden state are fp32.
+    x may be fp32 or bfloat16 embeddings (read as they are: half the bytes)."""
+    B, S, d = x.shape
+    ragged = LAYOUT == "ragged"
+    M = lens.N if ragged else B * S
+    offs = _ptr(lens.offs) if ragged else 0
+    dev = x.device
+    hd = d // nheads
+    m = packed.params
+    emb = m.embeddings
+    pos, typ = emb.position_embeddings.weight.detach(), emb.token_type_embeddings.weight.detach()[0]
+    if x.dtype == torch.bfloat16:
+        h = torch.empty((M, d), device=dev, dtype=torch.float32)
+        h_lo = torch.empty((M, d), device=dev, dtype=torch.float32)
+        _call("mts_embed_ln_fwd_bf16in", _ptr(x), x.stride(0), _ptr(pos), _ptr(typ), _ptr(emb.LayerNorm.weight.detach()),
+              _ptr(emb.LayerNorm.bias.detach()), B, S, d, LN_EPS, _ptr(h), _ptr(h_lo), d, _ptr(lens.dev) if ragged else 0, offs,
+              _stream())
+    else:
+        h, _, h_lo, _, _ = _ln(0, x, pos, typ, emb.LayerNorm.weight.detach(), emb.LayerNorm.bias.detach(), B, S, d, True, False,
+                               lens if ragged else None)
+    n_layers = len(m.encoder.layer)
+    for l in range(n_layers):
+        lyr = m.encoder.layer[l]
+        ent = packed.packed_bf16(l)
+        F = lyr.intermediate.dense.out_features
+        qkv = torch.empty((M, 3 * d), device=dev, dtype=torch.bfloat16)
+        _call("mts_gemm_bf16p_out16", _ptr(h_lo), _ptr(ent["wqkv_bf"]), _ptr(ent["bqkv"]), _ptr(qkv), M, 3 * d, d, 3 * d, _stream())
+        a_lo = torch.empty((M, d), device=dev, dtype=torch.float32)
+        _call("mts_band_attn_fwd_bf16", _ptr(qkv), 3 * d, M, _ptr(lens.dev), offs, B, S, nheads, hd, reaches[l], 0, _ptr(a_lo), d, 0,
+              _stream())
+        t = torch.empty((M, d), device=dev, dtype=torch.float32)
+        _call("mts_gemm_bf16p", _ptr(a_lo), _ptr(ent["wo_bf"]), _ptr(ent["bo"]), _ptr(t), M, d, d, d, 1, 0, _stream())
+        ln1 = lyr.attention.output.LayerNorm
+        y, _, y_lo, _, _ = _ln(1, t, h, None, ln1.weight.detach(), ln1.bias.detach(), M, 1, d, True, False)
+        kf = _pad32(F)
+        z_hl = torch.empty((2, M, kf), device=dev, dtype=torch.float32)
+        if kf == F and d <= 3072:
+            _call("mts_gemm_bf16p_gelu_pair", _ptr(y_lo), _ptr(ent["w1_bf"]), _ptr(ent["b1"]), _ptr(z_hl[0]), _ptr(z_hl[1]), M, F, d,
+                  _stream())
+        else:
+            zp = torch.empty((M, F), device=dev, dtype=torch.float32)
+            _call("mts_gemm_bf16p", _ptr(y_lo), _ptr(ent["w1_bf"]), _ptr(ent["b1"]), _ptr(zp), M, F, d, F, 1, 0, _stream())
+            _call("mts_gelu_split", _ptr(zp), F, M, F, kf, 0, _ptr(z_hl[0]), _ptr(z_hl[1]), _stream())
+        u = torch.empty((M, d), device=dev, dtype=torch.float32)
+        _call("mts_gemm_bf16p", _ptr(z_hl[1]), _ptr(ent["w2_bf"]), _ptr(ent["b2"]), _ptr(u), M, d, kf, d, 1, 0, _stream())
+        ln2 = lyr.output.LayerNorm
+        h, _, h_lo, _, _ = _ln(1, u, y, None, ln2.weight.detach(), ln2.bias.detach(), M, 1, d, l + 1 < n_layers, False)
+    if ragged:  # back to the caller's [B,S,d] layout, padded sentences zero
+        out = torch.empty((B, S, d), device=dev, dtype=torch.float32)
+        _call("mts_ragged_copy", _ptr(h), _ptr(out), _ptr(lens.dev), _ptr(lens.offs), B, S, d, 1, 0.0, _stream())
+        return out
+    return h.view(B, S, d)
+
+
 def encoder_forward(x, lens, packed: PackedEncoder, nheads, reaches, save, p_hidden=0.0, p_attn=0.0):
     """x [B,S,d] -> last hidden state [B,S,d].  `reaches[l]` = one-sided window of layer l.
     With save=True also returns what the backward pass needs.
@@ -363,6 +446,8 @@ def encoder_forward(x, lens, packed: PackedEncoder, nheads, reaches, save, p_hid
     B, S, d = x.shape
     ragged = LAYOUT == "ragged"
     M = lens.N if ragged else B * S
+    if not save and p_hidden == 0 and p_attn == 0 and _bf16_eligible(d, nheads):
+        return encoder_forward_bf16(x, lens, packed, nheads, reaches), None
     if not save and p_hidden == 0 and p_attn == 0 and not FOLD_RESIDUAL and _f16x3_eligible(M, d, 0, ops):
         return encoder_forward_f16(x, lens, packed, nheads, reaches), None
     offs = _ptr(lens.offs) if ragged else 0
@@ -492,7 +577,12 @@ class Longformer_Local_Attention(nn.Module):
         return self._packed
 
     def forward(self, src, lengths):
-        x = ops._check(src, "src")
+        if torch.is_tensor(src) and src.dtype == torch.bfloat16:   # bf16 embeddings: inference under ops.set_precision("bf16")
+            x = ops._check(src, "src", torch.bfloat16)
+            if ops.PRECISION != "bf16":
+                raise TypeError("src: bfloat16 embeddings belong to the bf16 path (ops.set_precision('bf16')); the fp32 path takes fp32")
+        else:
+            x = ops._check(src, "src")
         if x.dim() != 3 or x.shape[2] != self.d_model:
             raise ValueError(f"expected [B, S, {self.d_model}] embeddings, got {tuple(x.shape)}")
         if x.shape[1] + 2 > self.max_positions:
@@ -506,7 +596,11 @@ class Longformer_Local_Attention(nn.Module):
         packed = self.packed()
         params = packed.used_parameters()
         if not (torch.is_grad_enabled() and any(p.requires_grad for p in params)):  # inference: nothing saved
+            if x.dtype == torch.bfloat16 and not (p_hidden == 0 and p_attn == 0 and _bf16_eligible(self.d_model, self.nhead)):
+                x = x.float()   # a shape or dropout setting the bf16 encoder does not serve: the fp32 path, on the same values
             return encoder_forward(x, lens, packed, self.nhead, self.reaches, save=False, p_hidden=p_hidden, p_attn=p_attn)[0]
+        if x.dtype == torch.bfloat16:
+            raise NotImplementedError("bfloat16 embeddings serve inference only (ops.set_precision('bf16')): train in fp32")
         return EncoderFn.apply(x, lens, packed, self.nhead, self.reaches, p_hidden, p_attn, *params)
 
 
