@@ -154,21 +154,35 @@ def _rows_ok(x, name, B, T):
     return x
 
 
+def _packs_by_8(x1, x2):
+    """The packed-operand-only kernels move 8 elements per 16-byte access: every width a multiple of 8, every batch stride
+    and source pointer on 16 bytes."""
+    return all(x.shape[2] % 8 == 0 and x.stride(0) * x.element_size() % 16 == 0 and x.data_ptr() % 16 == 0
+               for x in (x1, x2) if x is not None)
+
+
 def pack_rows_packed(x1, x2, B, T):
     """bf16 path: [x1[b,:T] | x2[b,:T]] -> the packed operand alone [B*T, pad32(D1+D2)].  The sources may be fp32 or -- embeddings
-    stored and shipped as bf16 -- bfloat16 tensors."""
+    stored and shipped as bf16 -- bfloat16 tensors, of any width: sources the 8-wide kernels cannot take are packed by the
+    element-wise kernel, bf16 ones widened to fp32 first (exact)."""
+    if x2 is not None and x2.dtype != x1.dtype:
+        raise TypeError("both modalities must have the same dtype")
     D1 = x1.shape[2]
     D2 = 0 if x2 is None else x2.shape[2]
     kp = _pad32(D1 + D2)
     lo = torch.empty((B * T, kp), device=x1.device, dtype=torch.float32)
+    by8 = _packs_by_8(x1, x2)
     if x1.dtype == torch.bfloat16:
-        if x2 is not None and x2.dtype != torch.bfloat16:
-            raise TypeError("both modalities must have the same dtype")
-        _call("mts_pack_rows_bf16in", _ptr(x1), x1.stride(0), D1, _ptr(x2), 0 if x2 is None else x2.stride(0), D2, B, T, kp,
-              _ptr(lo), _stream())
-    else:
-        _call("mts_pack_rows_split", _ptr(x1), x1.stride(0), D1, _ptr(x2), 0 if x2 is None else x2.stride(0), D2, B, T, kp,
-              0, _ptr(lo), _stream())
+        if by8:
+            _call("mts_pack_rows_bf16in", _ptr(x1), x1.stride(0), D1, _ptr(x2), 0 if x2 is None else x2.stride(0), D2, B, T, kp,
+                  _ptr(lo), _stream())
+            return lo
+        x1, x2 = x1[:B, :T].float(), (None if x2 is None else x2[:B, :T].float())
+        by8 = _packs_by_8(x1, x2)
+    # the element-wise kernel writes the fp32 operand too: a scratch `hi`, dropped
+    hi = None if by8 else torch.empty_like(lo)
+    _call("mts_pack_rows_split", _ptr(x1), x1.stride(0), D1, _ptr(x2), 0 if x2 is None else x2.stride(0), D2, B, T, kp,
+          _ptr(hi), _ptr(lo), _stream())
     return lo
 
 
