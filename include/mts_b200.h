@@ -192,7 +192,10 @@ int mts_pack_rows_bf16in(const void *src1, int64_t bstride1, int D1, const void 
  *                              S = Q K^T and O += P V as kind::f16 tcgen05.mma with fp32 accumulation, fp32 softmax, P rounded
  *                              to bf16.  Same masks and padded-query zeros as mts_band_attn_fwd; S <= 4094.  Outputs: out fp32
  *                              [rows, nheads*hd] and / or out_lo [rows, Kp] (the packed operand of mts_gemm_bf16p, Kp ==
- *                              nheads*hd); lse [B, nheads, S] or NULL.  Head dims 16, 32, 64, 112, 128 (else MTS_E_UNSUPPORTED). */
+ *                              nheads*hd); lse [B, nheads, S] or NULL.  Head dims: those of mts_band_attn_bf16_supported (else
+ *                              MTS_E_UNSUPPORTED).
+ *   mts_band_attn_bf16_supported : nonzero for the head dims mts_band_attn_fwd_bf16 serves: 16, 32, 64, 112, 128 and 144 .. 256
+ *                              in steps of 16. */
 int mts_gemm_bf16p_out16(const float *A_lo, const float *B_lo, const float *bias, void *C, int M, int N, int Kp, int64_t ldc,
                          void *stream);
 int mts_gemm_bf16p_gelu_pair(const float *A_lo, const float *B_lo, const float *bias, float *C, float *C_lo, int M, int N, int Kp,
@@ -202,6 +205,7 @@ int mts_embed_ln_fwd_bf16in(const void *x, int64_t x_bstride, const float *pos, 
                             const int32_t *lengths, const int32_t *offsets, void *stream);
 int mts_band_attn_fwd_bf16(const void *qkv, int64_t ld, int64_t rows, const int32_t *lengths, const int32_t *offsets, int B,
                            int S, int nheads, int hd, int w, float *out, float *out_lo, int Kp, float *lse, void *stream);
+int mts_band_attn_bf16_supported(int hd);
 
 /* Profiling hook of the tensor-core recurrence: installs (or, with NULL, removes) a device buffer of 4 x 12 int64
  * into which CTA 0 writes clock64() stamps of the phases of steps 8..11 (see csrc/lstm_rec_tc.cu). */
@@ -356,7 +360,7 @@ int mts_gelu_split(const float *src, int64_t ld, int rows, int cols, int Kp, flo
 /* LongformerSelfAttention (:481-639; sliding chunks :758-867) for all-local attention:
  *   qkv [B*S, ld] rows = [q | k | v] (each nheads*hd wide, head-major), q NOT yet scaled (the kernel divides by
  *   sqrt(hd) as HF does at :513); token i attends to j with |i-j| <= w and j < len_b; softmax in fp32;
- *   rows i >= len_b give exact zeros (:578).  hd % 4 == 0, hd <= 128.
+ *   rows i >= len_b give exact zeros (:578).  hd % 4 == 0, hd <= 256.
  *   out [B*S, nheads*hd] and/or its TF32 halves out_hi/out_lo [B*S,Kp] (Kp == nheads*hd);
  *   lse [B,nheads,S] or NULL: log-sum-exp of every query row, saved for the backward pass. */
 int mts_band_attn_fwd(const float *qkv, int64_t ld, const int32_t *lengths, const int32_t *offsets, int B, int S,
@@ -368,8 +372,8 @@ int mts_band_attn_fwd(const float *qkv, int64_t ld, const int32_t *lengths, cons
 int mts_band_attn_fwd_mma(const float *qkv, int64_t ld, const int32_t *lengths, const int32_t *offsets, int B, int S,
                           int nheads, int hd, int w, float *out, float *out_hi, float *out_lo, int Kp, float *lse,
                           void *stream);
-/* The CUDA-core (packed FFMA2) kernel: any head dim that is a multiple of 4 and <= 128.  mts_band_attn_fwd falls back
- * to it for head dims the tcgen05 kernel is not instantiated for. */
+/* The CUDA-core (packed FFMA2) kernel: any head dim that is a multiple of 4 and <= 256.  mts_band_attn_fwd falls back
+ * to it for head dims the tcgen05 kernel is not instantiated for (among them every head dim above 128). */
 int mts_band_attn_fwd_simt(const float *qkv, int64_t ld, const int32_t *lengths, const int32_t *offsets, int B, int S,
                            int nheads, int hd, int w, float *out, float *out_hi, float *out_lo, int Kp, float *lse,
                            void *stream);
@@ -400,7 +404,7 @@ int mts_embed_bwd(const float *dpre, int B, int S, int d, float *dpos, const int
                   void *stream);
 /* Banded attention backward: qkv, lse as in the forward call, o = forward output [B*S, nheads*hd], d_o its
  * gradient -> dqkv [B*S, ld] = [dq | dk | dv] (dq already includes the 1/sqrt(hd) factor), zero at padded rows.
- * delta_ws: B*nheads*S floats of scratch. */
+ * delta_ws: B*nheads*S floats of scratch.  hd % 4 == 0, hd <= 256. */
 int mts_band_attn_bwd(const float *qkv, int64_t ld, const float *o, const float *d_o, const float *lse,
                       const int32_t *lengths, const int32_t *offsets, int B, int S, int nheads, int hd, int w, float *dqkv,
                       float *delta_ws, void *stream);

@@ -45,6 +45,7 @@ SIGNATURES = {
     "mts_gemm_bf16p_gelu_pair": (c_int, [_P, _P, _P, _P, _P, c_int, c_int, c_int, _P]),
     "mts_embed_ln_fwd_bf16in": (c_int, [_P, c_int64, _P, _P, _P, _P, c_int, c_int, c_int, c_float, _P, _P, c_int, _P, _P, _P]),
     "mts_band_attn_fwd_bf16": (c_int, [_P, c_int64, c_int64, _P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P, c_int, _P, _P]),
+    "mts_band_attn_bf16_supported": (c_int, [c_int]),
     "mts_pack_rows_bf16in": (c_int, [_P, c_int64, c_int, _P, c_int64, c_int, c_int, c_int, c_int, _P, _P]),
     "mts_debug_rec_profile": (c_int, [_P]),
     "mts_debug_rec_profile_h3": (c_int, [_P]),

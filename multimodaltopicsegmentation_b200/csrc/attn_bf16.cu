@@ -14,7 +14,8 @@
 // memory (.ss form): the .ts form would need the worker warps to stage Q through registers into tensor memory (~5.5 k cycles per
 // item in attn_tc.cu), while the TMA lands the tile in shared memory with no worker involvement; S costs HD / 16 MMAs per key tile.
 //
-// Tensor memory (512 columns): S tiles [128,192) [192,256) fp32 | P tiles [256,288) [288,320) bf16 pairs | O [384, 384+HD).
+// Tensor memory (512 columns): S tiles [128,192) [192,256) fp32 | P tiles [256,288) [288,320) bf16 pairs | O [384, 384+HD);
+// heads wider than 128 move S to [0,128) and P to [128,192) so that O [256, 256+HD) fits (512 columns at HD 256).
 // Warps: 8 uniform worker warps (softmax + epilogue, as in attn_tc.cu), warp 8 MMA issuer, warps 9 / 10 / 11 TMA loaders of
 // K / V / Q.  Per key tile a worker warp only reads S, masks, exchanges row maxima with its partner warp and writes P.
 #include <stdlib.h>
@@ -24,11 +25,10 @@
 namespace mts {
 namespace atc {
 
-constexpr uint32_t B16_COL_S = 128, B16_COL_P = 256, B16_COL_O = 384;
-
 template <int HD>
 struct Cfg16 {
-  static_assert(HD % 16 == 0 && HD >= 16 && HD <= 128, "head dim: multiple of 16, at most 128");
+  static_assert(HD % 16 == 0 && HD >= 16 && HD <= 256, "head dim: multiple of 16, at most 256");
+  static constexpr uint32_t COL_S = HD <= 128 ? 128 : 0, COL_P = HD <= 128 ? 256 : 128, COL_O = HD <= 128 ? 384 : 256;
   static constexpr int NP = (HD + 63) / 64;    // 64-column (128-byte) planes of a bf16 operand
   static constexpr int NC = HD / 16;           // 16-column chunks per row
   static constexpr int Q_BYTES = NP * BQ * 128;
@@ -45,6 +45,7 @@ struct Cfg16 {
   static constexpr int USED = OFF_META + 2 * META_B * 4;
   // every CTA allocates all 512 TMEM columns, so two CTAs must never share an SM: ask for more than half its shared memory
   static constexpr int SMEM = (USED + 1024) > 120 * 1024 ? (USED + 1024) : 120 * 1024;
+  static_assert(SMEM <= 227 * 1024, "shared memory of one CTA");
 };
 
 enum { C_QFULL = 0, C_QFREE, C_KFULL0, C_KFULL1, C_KEMPTY0, C_KEMPTY1, C_VFULL0, C_VFULL1, C_VEMPTY0, C_VEMPTY1,
@@ -134,7 +135,7 @@ __global__ void __launch_bounds__(THREADS, 1)
           bar_wait(BAR(C_SFULL0 + buf), (tile_g >> 1) & 1);
           tc::tc_fence_after();
           float s[32];
-          tmem_ld32_nowait(trow + B16_COL_S + 64 * buf + 32 * ch, s);
+          tmem_ld32_nowait(trow + C::COL_S + 64 * buf + 32 * ch, s);
           tmem_wait_ld();
           // 16-key blocks that no row of this warp can see are not evaluated: their probabilities are stored as zeros
           unsigned live = 0;
@@ -171,11 +172,11 @@ __global__ void __launch_bounds__(THREADS, 1)
             for (int c = ch; c < C::NC; c += 2) {
               float v[16];
               uint32_t u[16];
-              tmem_ld16_nowait(trow + B16_COL_O + 16 * c, v);
+              tmem_ld16_nowait(trow + C::COL_O + 16 * c, v);
               tmem_wait_ld();
 #pragma unroll
               for (int e = 0; e < 16; ++e) u[e] = __float_as_uint(v[e] * alpha);
-              tmem_st16(trow + B16_COL_O + 16 * c, u);
+              tmem_st16(trow + C::COL_O + 16 * c, u);
             }
           }
           const float mb = (m_run == -INFINITY) ? 0.0f : -m_run * LOG2E;
@@ -196,7 +197,7 @@ __global__ void __launch_bounds__(THREADS, 1)
             }
           }
           // P buffer `buf` was last read by the P V of tile tile_g - 2, complete before this tile's S (see C_SFULL above)
-          tmem_st16(trow + B16_COL_P + 32 * buf + 16 * ch, pb);
+          tmem_st16(trow + C::COL_P + 32 * buf + 16 * ch, pb);
           l_run += (ps4[0] + ps4[1]) + (ps4[2] + ps4[3]);
           tc::tmem_wait_st();
           tc::tc_fence_before();
@@ -222,7 +223,7 @@ __global__ void __launch_bounds__(THREADS, 1)
 #pragma unroll
           for (int e = 0; e < 16; ++e) v[e] = 0.0f;
           if (it.active) {
-            tmem_ld16_nowait(trow + B16_COL_O + 16 * c, v);
+            tmem_ld16_nowait(trow + C::COL_O + 16 * c, v);
             tmem_wait_ld();
           }
 #pragma unroll
@@ -313,7 +314,7 @@ __global__ void __launch_bounds__(THREADS, 1)
           const uint32_t kb = s_cnt & 1;
           bar_wait(BAR(C_KFULL0 + kb), (s_cnt >> 1) & 1);
           tc::tc_fence_after();
-          const uint32_t d_s = tb + B16_COL_S + 64 * (s_cnt & 1);
+          const uint32_t d_s = tb + C::COL_S + 64 * (s_cnt & 1);
 #pragma unroll
           for (int ks = 0; ks < HD / 16; ++ks) {   // K = 16 bf16 = 32 bytes per MMA inside a 128-byte swizzle row
             const uint64_t ad = desc_add(q_desc, (uint32_t)((ks >> 2) * (BQ * 128) + (ks & 3) * 32));
@@ -338,11 +339,11 @@ __global__ void __launch_bounds__(THREADS, 1)
         bar_wait(BAR(C_VFULL0 + buf), (tile_g >> 1) & 1);
         if (t == 0) bar_wait(BAR(C_OFREE), (item_g & 1) ^ 1);   // the previous item's epilogue has read O
         tc::tc_fence_after();
-        const uint32_t d_o = tb + B16_COL_O;
+        const uint32_t d_o = tb + C::COL_O;
 #pragma unroll
         for (int kg = 0; kg < KT / 16; ++kg) {   // 16 keys = 16 rows of 128 bytes of the V tile per MMA
           const uint64_t bd = desc_add(v_desc, (uint32_t)(buf * C::T_BYTES + kg * 2048));
-          if (leader) tc::umma_bf16_ts(d_o, tb + B16_COL_P + 32 * buf + 8 * kg, bd, id_o, (t | kg) != 0);
+          if (leader) tc::umma_bf16_ts(d_o, tb + C::COL_P + 32 * buf + 8 * kg, bd, id_o, (t | kg) != 0);
         }
         if (leader) {
           tc::umma_commit(BAR(C_VEMPTY0 + buf));
@@ -401,6 +402,10 @@ static int launch_bf16(const void *qkv, int64_t ld, int64_t rows, const int32_t 
 
 using namespace mts;
 
+extern "C" int mts_band_attn_bf16_supported(int hd) {
+  return hd == 16 || hd == 32 || hd == 64 || hd == 112 || hd == 128 || (hd >= 144 && hd <= 256 && hd % 16 == 0);
+}
+
 extern "C" int mts_band_attn_fwd_bf16(const void *qkv, int64_t ld, int64_t rows, const int32_t *lengths, const int32_t *offsets,
                                       int B, int S, int nheads, int hd, int w, float *out, float *out_lo, int Kp, float *lse,
                                       void *stream) {
@@ -411,15 +416,17 @@ extern "C" int mts_band_attn_fwd_bf16(const void *qkv, int64_t ld, int64_t rows,
   MTS_REQUIRE(((uintptr_t)qkv & 15) == 0 && ((uintptr_t)out & 15) == 0 && ((uintptr_t)out_lo & 15) == 0, MTS_E_BADARG,
               "band_attn_fwd_bf16: buffers must be 16-byte aligned");
   MTS_REQUIRE(!out_lo || Kp == nheads * hd, MTS_E_UNSUPPORTED, "band_attn_fwd_bf16: the packed output needs Kp == model width");
+  MTS_REQUIRE(mts_band_attn_bf16_supported(hd), MTS_E_UNSUPPORTED,
+              "band_attn_fwd_bf16: head dim must be one of 16, 32, 64, 112, 128 or 144 .. 256 in steps of 16");
   cudaStream_t st = (cudaStream_t)stream;
   switch (hd) {
-    case 16: return atc::launch_bf16<16>(qkv, ld, rows, lengths, offsets, B, S, nheads, w, out, out_lo, lse, st);
-    case 32: return atc::launch_bf16<32>(qkv, ld, rows, lengths, offsets, B, S, nheads, w, out, out_lo, lse, st);
-    case 64: return atc::launch_bf16<64>(qkv, ld, rows, lengths, offsets, B, S, nheads, w, out, out_lo, lse, st);
-    case 112: return atc::launch_bf16<112>(qkv, ld, rows, lengths, offsets, B, S, nheads, w, out, out_lo, lse, st);
-    case 128: return atc::launch_bf16<128>(qkv, ld, rows, lengths, offsets, B, S, nheads, w, out, out_lo, lse, st);
+#define MTS_BF16_HD(H) \
+  case H: return atc::launch_bf16<H>(qkv, ld, rows, lengths, offsets, B, S, nheads, w, out, out_lo, lse, st);
+    MTS_BF16_HD(16) MTS_BF16_HD(32) MTS_BF16_HD(64) MTS_BF16_HD(112) MTS_BF16_HD(128)
+    MTS_BF16_HD(144) MTS_BF16_HD(160) MTS_BF16_HD(176) MTS_BF16_HD(192) MTS_BF16_HD(208) MTS_BF16_HD(224) MTS_BF16_HD(240)
+    MTS_BF16_HD(256)
+#undef MTS_BF16_HD
     default: break;
   }
-  set_error("band_attn_fwd_bf16: head dim must be one of 16, 32, 64, 112, 128");
-  return MTS_E_UNSUPPORTED;
+  return MTS_E_UNSUPPORTED;   // not reached: mts_band_attn_bf16_supported lists exactly the instantiations above
 }

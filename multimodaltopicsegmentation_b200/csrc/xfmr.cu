@@ -226,7 +226,8 @@ __global__ void __launch_bounds__(256) gelu_split_v8_kernel(const float *__restr
 //   phases 1 + 2  S = Q K^T and the running softmax, warp-local: warp = 4 queries x the 64 keys of the tile (thread =
 //             4 queries x 2 keys, float4 along the head dimension, FFMA2); row max / exp / sum by shuffles, the four rows
 //             interleaved; running statistics in registers; P and the rescale factors go to shared memory
-//   phase 3   O = alpha O + P V   warp = 4 float4 head columns, thread = 4 queries x 1 float4 column (FFMA2)
+//   phase 3   O = alpha O + P V   warp = 4 float4 head columns, thread = 4 queries x 1 float4 column (FFMA2); heads wider
+//             than 128 (NCW = 2): thread = 4 queries x the float4 columns cg and cg + 32, sharing the P loads
 // Three block-wide barriers per tile; K / V tiles by cp.async.
 // Shared rows are padded to a stride = 4 (mod 8) words so that 8 consecutive rows read as float4 hit
 // 8 distinct bank groups.
@@ -240,7 +241,8 @@ static size_t ba_smem_bytes(int hd) {
 
 // DROP: dropout on the probabilities (training): the weights of P V are p * keep / (1 - p_drop), the softmax denominator
 // and the saved log-sum-exp stay those of the undropped probabilities (attn_keep_scale, common.cuh).
-template <bool DROP>
+// NCW: float4 head columns per phase-3 thread, 1 for hd <= 128, 2 for 128 < hd <= 256.
+template <bool DROP, int NCW>
 __global__ void __launch_bounds__(BA_THREADS, 2)
     band_attn_fwd_kernel(const float *__restrict__ qkv, int64_t ld, const int32_t *__restrict__ lengths,
                          const int32_t *__restrict__ offsets, int S, int nheads, int hd, int w,
@@ -267,20 +269,28 @@ __global__ void __launch_bounds__(BA_THREADS, 2)
   // the 8 lane groups (lane >> 2) take 8 consecutive P rows, the 4 lanes of a group 4 consecutive 16-byte V columns;
   // warp = 4 float4 head columns, thread = 4 queries (qgrp + 8r) x 1 float4 column.
   const int qgrp = lane >> 2;
-  const int cg = 4 * warp + (lane & 3);   // phase 3 / output: my float4 column of the head
+  const int cg = 4 * warp + (lane & 3);   // phase 3 / output: my float4 column of the head (and cg + 32 .. when NCW > 1)
   const bool pv_thread = cg < nv;
+  // column of chunk c; a thread whose cg + 32 c lies past the head computes the last column again and does not store it
+  auto col = [&](int c) { return c == 0 ? cg : min(cg + 32 * c, nv - 1); };
+  auto col_ok = [&](int c) { return c == 0 || cg + 32 * c < nv; };
 
   if (q0 >= len) {  // whole block is padding: exact zeros
     if (pv_thread) {
 #pragma unroll
-      for (int r = 0; r < 4; ++r) {
-        const int i = q0 + qgrp + 8 * r;
-        if (i < Sq) {
-          const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (out) reinterpret_cast<float4 *>(out + (row0 + i) * d + head * hd)[cg] = z;
-          if (out_hi) {
-            reinterpret_cast<float4 *>(out_hi + (row0 + i) * Kp + head * hd)[cg] = z;
-            corr_store4(out_lo + (row0 + i) * Kp, head * hd + 4 * cg, z, 0);
+      for (int c = 0; c < NCW; ++c) {
+        if (!col_ok(c)) continue;
+        const int cc = col(c);
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {
+          const int i = q0 + qgrp + 8 * r;
+          if (i < Sq) {
+            const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (out) reinterpret_cast<float4 *>(out + (row0 + i) * d + head * hd)[cc] = z;
+            if (out_hi) {
+              reinterpret_cast<float4 *>(out_hi + (row0 + i) * Kp + head * hd)[cc] = z;
+              corr_store4(out_lo + (row0 + i) * Kp, head * hd + 4 * cc, z, 0);
+            }
           }
         }
       }
@@ -303,9 +313,11 @@ __global__ void __launch_bounds__(BA_THREADS, 2)
 #pragma unroll
   for (int a = 0; a < 4; ++a) { m_run[a] = -INFINITY; l_run[a] = 0.0f; }
 
-  float2 o2[4][2];   // 4 queries x (columns 0-1, columns 2-3) of my float4 head column
+  float2 o2[NCW][4][2];   // per float4 head column: 4 queries x (columns 0-1, columns 2-3)
 #pragma unroll
-  for (int r = 0; r < 4; ++r) o2[r][0] = o2[r][1] = make_float2(0.0f, 0.0f);
+  for (int c = 0; c < NCW; ++c)
+#pragma unroll
+    for (int r = 0; r < 4; ++r) o2[c][r][0] = o2[c][r][1] = make_float2(0.0f, 0.0f);
 
   const int kbeg = max(0, q0 - w), kend = min(len, q0 + BA_BQ + w);
 
@@ -408,8 +420,11 @@ __global__ void __launch_bounds__(BA_THREADS, 2)
 #pragma unroll
       for (int r = 0; r < 4; ++r) {
         const float al = al_s[qgrp + 8 * r];
-        o2[r][0] = __fmul2_rn(o2[r][0], make_float2(al, al));
-        o2[r][1] = __fmul2_rn(o2[r][1], make_float2(al, al));
+#pragma unroll
+        for (int c = 0; c < NCW; ++c) {
+          o2[c][r][0] = __fmul2_rn(o2[c][r][0], make_float2(al, al));
+          o2[c][r][1] = __fmul2_rn(o2[c][r][1], make_float2(al, al));
+        }
       }
 #pragma unroll 4
       for (int k4 = 0; k4 < BA_TK / 4; ++k4) {
@@ -418,13 +433,16 @@ __global__ void __launch_bounds__(BA_THREADS, 2)
         for (int r = 0; r < 4; ++r) p[r] = reinterpret_cast<const float4 *>(Ps + (qgrp + 8 * r) * BA_PS)[k4];
 #pragma unroll
         for (int kk = 0; kk < 4; ++kk) {
-          const float4 vv = reinterpret_cast<const float4 *>(Vs + (4 * k4 + kk) * RS)[cg];
 #pragma unroll
-          for (int r = 0; r < 4; ++r) {
-            const float pk = kk == 0 ? p[r].x : kk == 1 ? p[r].y : kk == 2 ? p[r].z : p[r].w;
-            const float2 pk2 = make_float2(pk, pk);
-            o2[r][0] = __ffma2_rn(pk2, make_float2(vv.x, vv.y), o2[r][0]);
-            o2[r][1] = __ffma2_rn(pk2, make_float2(vv.z, vv.w), o2[r][1]);
+          for (int c = 0; c < NCW; ++c) {
+            const float4 vv = reinterpret_cast<const float4 *>(Vs + (4 * k4 + kk) * RS)[col(c)];
+#pragma unroll
+            for (int r = 0; r < 4; ++r) {
+              const float pk = kk == 0 ? p[r].x : kk == 1 ? p[r].y : kk == 2 ? p[r].z : p[r].w;
+              const float2 pk2 = make_float2(pk, pk);
+              o2[c][r][0] = __ffma2_rn(pk2, make_float2(vv.x, vv.y), o2[c][r][0]);
+              o2[c][r][1] = __ffma2_rn(pk2, make_float2(vv.z, vv.w), o2[c][r][1]);
+            }
           }
         }
       }
@@ -439,18 +457,23 @@ __global__ void __launch_bounds__(BA_THREADS, 2)
 
   if (pv_thread) {
 #pragma unroll
-    for (int r = 0; r < 4; ++r) {
-      const int i = q0 + qgrp + 8 * r;
-      if (i >= Sq) continue;
-      float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (i < len) {
-        const float inv = 1.0f / l_s[qgrp + 8 * r];
-        v = make_float4(o2[r][0].x * inv, o2[r][0].y * inv, o2[r][1].x * inv, o2[r][1].y * inv);
-      }
-      if (out) reinterpret_cast<float4 *>(out + (row0 + i) * d + head * hd)[cg] = v;
-      if (out_hi) {
-        reinterpret_cast<float4 *>(out_hi + (row0 + i) * Kp + head * hd)[cg] = v;
-        corr_store4(out_lo + (row0 + i) * Kp, head * hd + 4 * cg, v, 0);
+    for (int c = 0; c < NCW; ++c) {
+      if (!col_ok(c)) continue;
+      const int cc = col(c);
+#pragma unroll
+      for (int r = 0; r < 4; ++r) {
+        const int i = q0 + qgrp + 8 * r;
+        if (i >= Sq) continue;
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (i < len) {
+          const float inv = 1.0f / l_s[qgrp + 8 * r];
+          v = make_float4(o2[c][r][0].x * inv, o2[c][r][0].y * inv, o2[c][r][1].x * inv, o2[c][r][1].y * inv);
+        }
+        if (out) reinterpret_cast<float4 *>(out + (row0 + i) * d + head * hd)[cc] = v;
+        if (out_hi) {
+          reinterpret_cast<float4 *>(out_hi + (row0 + i) * Kp + head * hd)[cc] = v;
+          corr_store4(out_lo + (row0 + i) * Kp, head * hd + 4 * cc, v, 0);
+        }
       }
     }
   }
@@ -844,13 +867,36 @@ extern "C" int mts_band_attn_fwd(const float *qkv, int64_t ld, const int32_t *le
   return mts_band_attn_fwd_simt(qkv, ld, lengths, offsets, B, S, nheads, hd, w, out, out_hi, out_lo, Kp, lse, stream);
 }
 
+template <int NCW>
+static int band_attn_fwd_launch(const float *qkv, int64_t ld, const int32_t *lengths, const int32_t *offsets, int B, int S,
+                                int nheads, int hd, int w, float *out, float *out_hi, float *out_lo, int Kp, float *lse,
+                                float p_drop, uint64_t seed, void *stream) {
+  const size_t smem = ba_smem_bytes(hd);
+  const dim3 grid((S + BA_BQ - 1) / BA_BQ, nheads, B);
+  if (p_drop > 0.0f) {
+    MTS_CUDA(cudaFuncSetAttribute(band_attn_fwd_kernel<true, NCW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    band_attn_fwd_kernel<true, NCW><<<grid, BA_THREADS, smem, (cudaStream_t)stream>>>(
+        qkv, ld, lengths, offsets, S, nheads, hd, w, out, out_hi, out_lo, Kp, lse, attn_drop_p24(p_drop), 1.0f / (1.0f - p_drop), seed);
+  } else {
+    MTS_PER_DEVICE(size_t, smem_set);   // one per instantiation and device
+    if (smem > smem_set) {
+      MTS_CUDA(cudaFuncSetAttribute(band_attn_fwd_kernel<false, NCW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      smem_set = smem;
+    }
+    band_attn_fwd_kernel<false, NCW><<<grid, BA_THREADS, smem, (cudaStream_t)stream>>>(qkv, ld, lengths, offsets, S, nheads, hd, w,
+                                                                                      out, out_hi, out_lo, Kp, lse, 0u, 1.0f, 0ull);
+  }
+  MTS_LAUNCH_CHECK();
+  return 0;
+}
+
 static int band_attn_fwd_simt_impl(const float *qkv, int64_t ld, const int32_t *lengths, const int32_t *offsets, int B, int S,
                                    int nheads, int hd, int w, float *out, float *out_hi, float *out_lo, int Kp, float *lse,
                                    float p_drop, uint64_t seed, void *stream) {
   MTS_REQUIRE(qkv && lengths && (out || out_hi), MTS_E_BADARG, "band_attn_fwd: null pointer");
   MTS_REQUIRE((out_hi == nullptr) == (out_lo == nullptr), MTS_E_BADARG, "band_attn_fwd: hi and lo go together");
   MTS_REQUIRE(B > 0 && S > 0 && nheads > 0 && hd > 0 && w >= 0, MTS_E_BADARG, "band_attn_fwd: bad shape");
-  MTS_REQUIRE(hd % 4 == 0 && hd <= 128, MTS_E_UNSUPPORTED, "band_attn_fwd: head dim must be a multiple of 4 and <= 128");
+  MTS_REQUIRE(hd % 4 == 0 && hd <= 256, MTS_E_UNSUPPORTED, "band_attn_fwd: head dim must be a multiple of 4 and <= 256");
   MTS_REQUIRE(ld % 4 == 0 && ld >= 3 * nheads * hd, MTS_E_BADARG, "band_attn_fwd: qkv row stride");
   MTS_REQUIRE(((uintptr_t)qkv & 15) == 0, MTS_E_BADARG, "band_attn_fwd: qkv must be 16-byte aligned");
   MTS_REQUIRE(!out_hi || (Kp % 32 == 0 && Kp >= nheads * hd), MTS_E_BADARG, "band_attn_fwd: Kp");
@@ -858,23 +904,9 @@ static int band_attn_fwd_simt_impl(const float *qkv, int64_t ld, const int32_t *
               "band_attn_fwd: the split output needs a model width that is a multiple of 32");
   MTS_REQUIRE(p_drop >= 0.0f && p_drop < 1.0f, MTS_E_BADARG, "band_attn_fwd: dropout probability must be in [0, 1)");
   MTS_REQUIRE(p_drop == 0.0f || S <= (1 << 20), MTS_E_UNSUPPORTED, "band_attn_fwd: dropout indices need S <= 2^20");
-  const size_t smem = ba_smem_bytes(hd);
-  const dim3 grid((S + BA_BQ - 1) / BA_BQ, nheads, B);
-  if (p_drop > 0.0f) {
-    MTS_CUDA(cudaFuncSetAttribute(band_attn_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    band_attn_fwd_kernel<true><<<grid, BA_THREADS, smem, (cudaStream_t)stream>>>(
-        qkv, ld, lengths, offsets, S, nheads, hd, w, out, out_hi, out_lo, Kp, lse, attn_drop_p24(p_drop), 1.0f / (1.0f - p_drop), seed);
-  } else {
-    MTS_PER_DEVICE(size_t, smem_set);
-    if (smem > smem_set) {
-      MTS_CUDA(cudaFuncSetAttribute(band_attn_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      smem_set = smem;
-    }
-    band_attn_fwd_kernel<false><<<grid, BA_THREADS, smem, (cudaStream_t)stream>>>(qkv, ld, lengths, offsets, S, nheads, hd, w, out,
-                                                                                 out_hi, out_lo, Kp, lse, 0u, 1.0f, 0ull);
-  }
-  MTS_LAUNCH_CHECK();
-  return 0;
+  if (hd > 128)
+    return band_attn_fwd_launch<2>(qkv, ld, lengths, offsets, B, S, nheads, hd, w, out, out_hi, out_lo, Kp, lse, p_drop, seed, stream);
+  return band_attn_fwd_launch<1>(qkv, ld, lengths, offsets, B, S, nheads, hd, w, out, out_hi, out_lo, Kp, lse, p_drop, seed, stream);
 }
 
 extern "C" int mts_band_attn_fwd_simt(const float *qkv, int64_t ld, const int32_t *lengths, const int32_t *offsets, int B,

@@ -145,6 +145,8 @@ __global__ void __launch_bounds__(256) embed_bwd_kernel(const float *__restrict_
 // tiles of the other side staged in shared memory, only tiles intersecting the band are read.
 //   dq kernel : own rows = queries; loops key tiles;   writes dq and delta[i] = sum_c dO[i,c] O[i,c]
 //   dkv kernel: own rows = keys;    loops query tiles; writes dk and dv (no atomics)
+// Output mapping (the P dK / P^T dO products): thread = 4 own rows x 1 float4 head column (cg = tid % nv, needs nv <= 32); heads
+// wider than 128 (NCW = 2): warp = 4 own rows, thread = the float4 columns cg and cg + 32 (cg = lane).
 // ---------------------------------------------------------------------------------------------------------
 constexpr int BB_OWN = 32, BB_TILE = 64, BB_THREADS = 256, BB_PS = BB_TILE + 4;
 
@@ -157,8 +159,11 @@ __device__ __forceinline__ float dot4(const float4 a, const float4 b, float acc)
 // DROP (both kernels): the forward pass weighted P V by p * m with m = keep / (1 - p_drop) (attn_keep_scale, regenerated here
 // from the seed): dV = (P .* M)^T dO, dP = M .* (dO V^T), dS = P .* (dP - delta) with delta = rowsum(dO .* O) as before
 // (sum_j P_ij dP_ij = dO_i . O_i holds with the dropped weights too).
-template <bool DROP>
-__global__ void __launch_bounds__(BB_THREADS, 2)
+// NCW (both kernels): float4 head columns per output thread, 1 for hd <= 128, 2 for 128 < hd <= 256.  The wide form keeps
+// twice the accumulators and gets the whole register file: from hd 136 on, the shared memory of either kernel allows only one CTA
+// per SM anyway.
+template <bool DROP, int NCW>
+__global__ void __launch_bounds__(BB_THREADS, NCW == 1 ? 2 : 1)
     band_attn_bwd_dq_kernel(const float *__restrict__ qkv, int64_t ld, const float *__restrict__ o,
                             const float *__restrict__ dO, const float *__restrict__ lse,
                             const int32_t *__restrict__ lengths, const int32_t *__restrict__ offsets, int S,
@@ -181,16 +186,23 @@ __global__ void __launch_bounds__(BB_THREADS, 2)
   // ragged layout (offsets != NULL): episode b owns rows offsets[b] .. offsets[b] + len - 1 and nothing beyond
   const int64_t row0 = offsets ? (int64_t)offsets[b] : (int64_t)b * S;
   const int Sq = offsets ? len : S;  // rows of this episode that exist in memory
-  const int cg = tid % nv, rg = tid / nv;
+  const int cg = NCW == 1 ? tid % nv : tid & 31, rg = NCW == 1 ? tid / nv : tid >> 5;
   const bool out_thread = rg < BB_OWN / 4;
+  // column of chunk c; a thread whose cg + 32 c lies past the head computes the last column again and does not store it
+  auto col = [&](int c) { return c == 0 ? cg : min(cg + 32 * c, nv - 1); };
+  auto col_ok = [&](int c) { return c == 0 || cg + 32 * c < nv; };
   const int64_t stat0 = ((int64_t)b * nheads + head) * S;
 
   if (q0 >= len) {
     if (out_thread) {
 #pragma unroll
-      for (int r = 0; r < 4; ++r) {
-        const int i = q0 + rg * 4 + r;
-        if (i < Sq) reinterpret_cast<float4 *>(dqkv + (row0 + i) * ld + head * hd)[cg] = make_float4(0.f, 0.f, 0.f, 0.f);
+      for (int c = 0; c < NCW; ++c) {
+        if (!col_ok(c)) continue;
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {
+          const int i = q0 + rg * 4 + r;
+          if (i < Sq) reinterpret_cast<float4 *>(dqkv + (row0 + i) * ld + head * hd)[col(c)] = make_float4(0.f, 0.f, 0.f, 0.f);
+        }
       }
     }
     if (tid < BB_OWN && q0 + tid < S) delta[stat0 + q0 + tid] = 0.0f;
@@ -225,11 +237,13 @@ __global__ void __launch_bounds__(BB_THREADS, 2)
     }
   }
 
-  float acc_o[4][4];
+  float acc_o[NCW][4][4];
 #pragma unroll
-  for (int r = 0; r < 4; ++r)
+  for (int n = 0; n < NCW; ++n)
 #pragma unroll
-    for (int c = 0; c < 4; ++c) acc_o[r][c] = 0.0f;
+    for (int r = 0; r < 4; ++r)
+#pragma unroll
+      for (int c = 0; c < 4; ++c) acc_o[n][r][c] = 0.0f;
 
   const int kbeg = max(0, q0 - w), kend = min(len, q0 + BB_OWN + w);
   const int qg = tid >> 4, kg = tid & 15;
@@ -291,14 +305,17 @@ __global__ void __launch_bounds__(BB_THREADS, 2)
         for (int r = 0; r < 4; ++r) p[r] = reinterpret_cast<const float4 *>(Ps + (rg * 4 + r) * BB_PS)[k4];
 #pragma unroll
         for (int kk = 0; kk < 4; ++kk) {
-          const float4 kv = reinterpret_cast<const float4 *>(Ks + (4 * k4 + kk) * RS)[cg];
 #pragma unroll
-          for (int r = 0; r < 4; ++r) {
-            const float pk = kk == 0 ? p[r].x : kk == 1 ? p[r].y : kk == 2 ? p[r].z : p[r].w;
-            acc_o[r][0] = fmaf(pk, kv.x, acc_o[r][0]);
-            acc_o[r][1] = fmaf(pk, kv.y, acc_o[r][1]);
-            acc_o[r][2] = fmaf(pk, kv.z, acc_o[r][2]);
-            acc_o[r][3] = fmaf(pk, kv.w, acc_o[r][3]);
+          for (int n = 0; n < NCW; ++n) {
+            const float4 kv = reinterpret_cast<const float4 *>(Ks + (4 * k4 + kk) * RS)[col(n)];
+#pragma unroll
+            for (int r = 0; r < 4; ++r) {
+              const float pk = kk == 0 ? p[r].x : kk == 1 ? p[r].y : kk == 2 ? p[r].z : p[r].w;
+              acc_o[n][r][0] = fmaf(pk, kv.x, acc_o[n][r][0]);
+              acc_o[n][r][1] = fmaf(pk, kv.y, acc_o[n][r][1]);
+              acc_o[n][r][2] = fmaf(pk, kv.z, acc_o[n][r][2]);
+              acc_o[n][r][3] = fmaf(pk, kv.w, acc_o[n][r][3]);
+            }
           }
         }
       }
@@ -306,18 +323,23 @@ __global__ void __launch_bounds__(BB_THREADS, 2)
   }
   if (out_thread) {
 #pragma unroll
-    for (int r = 0; r < 4; ++r) {
-      const int i = q0 + rg * 4 + r;
-      if (i >= Sq) continue;
-      float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (i < len) v = make_float4(acc_o[r][0] / scale, acc_o[r][1] / scale, acc_o[r][2] / scale, acc_o[r][3] / scale);
-      reinterpret_cast<float4 *>(dqkv + (row0 + i) * ld + head * hd)[cg] = v;
+    for (int n = 0; n < NCW; ++n) {
+      if (!col_ok(n)) continue;
+#pragma unroll
+      for (int r = 0; r < 4; ++r) {
+        const int i = q0 + rg * 4 + r;
+        if (i >= Sq) continue;
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (i < len)
+          v = make_float4(acc_o[n][r][0] / scale, acc_o[n][r][1] / scale, acc_o[n][r][2] / scale, acc_o[n][r][3] / scale);
+        reinterpret_cast<float4 *>(dqkv + (row0 + i) * ld + head * hd)[col(n)] = v;
+      }
     }
   }
 }
 
-template <bool DROP>
-__global__ void __launch_bounds__(BB_THREADS, 2)
+template <bool DROP, int NCW>
+__global__ void __launch_bounds__(BB_THREADS, NCW == 1 ? 2 : 1)
     band_attn_bwd_dkv_kernel(const float *__restrict__ qkv, int64_t ld, const float *__restrict__ dO,
                              const float *__restrict__ lse, const float *__restrict__ delta,
                              const int32_t *__restrict__ lengths, const int32_t *__restrict__ offsets, int S,
@@ -341,15 +363,20 @@ __global__ void __launch_bounds__(BB_THREADS, 2)
   // ragged layout (offsets != NULL): episode b owns rows offsets[b] .. offsets[b] + len - 1 and nothing beyond
   const int64_t row0 = offsets ? (int64_t)offsets[b] : (int64_t)b * S;
   const int Sq = offsets ? len : S;  // rows of this episode that exist in memory
-  const int cg = tid % nv, rg = tid / nv;
+  const int cg = NCW == 1 ? tid % nv : tid & 31, rg = NCW == 1 ? tid / nv : tid >> 5;
   const bool out_thread = rg < BB_OWN / 4;
+  // column of chunk c; a thread whose cg + 32 c lies past the head computes the last column again and does not store it
+  auto col = [&](int c) { return c == 0 ? cg : min(cg + 32 * c, nv - 1); };
+  auto col_ok = [&](int c) { return c == 0 || cg + 32 * c < nv; };
   const int64_t stat0 = ((int64_t)b * nheads + head) * S;
 
-  float dk[4][4], dv[4][4];
+  float dk[NCW][4][4], dv[NCW][4][4];
 #pragma unroll
-  for (int r = 0; r < 4; ++r)
+  for (int n = 0; n < NCW; ++n)
 #pragma unroll
-    for (int c = 0; c < 4; ++c) { dk[r][c] = 0.0f; dv[r][c] = 0.0f; }
+    for (int r = 0; r < 4; ++r)
+#pragma unroll
+      for (int c = 0; c < 4; ++c) { dk[n][r][c] = 0.0f; dv[n][r][c] = 0.0f; }
 
   if (k0 < len) {
     for (int idx = tid; idx < BB_OWN * nv; idx += BB_THREADS) {
@@ -433,16 +460,19 @@ __global__ void __launch_bounds__(BB_THREADS, 2)
           }
 #pragma unroll
           for (int kk = 0; kk < 4; ++kk) {
-            const float4 gv = reinterpret_cast<const float4 *>(Gs + (4 * q4 + kk) * RS)[cg];
-            const float4 qv = reinterpret_cast<const float4 *>(Qs + (4 * q4 + kk) * RS)[cg];
 #pragma unroll
-            for (int r = 0; r < 4; ++r) {
-              const float pk = kk == 0 ? p[r].x : kk == 1 ? p[r].y : kk == 2 ? p[r].z : p[r].w;
-              const float sk = kk == 0 ? s[r].x : kk == 1 ? s[r].y : kk == 2 ? s[r].z : s[r].w;
-              dv[r][0] = fmaf(pk, gv.x, dv[r][0]); dv[r][1] = fmaf(pk, gv.y, dv[r][1]);
-              dv[r][2] = fmaf(pk, gv.z, dv[r][2]); dv[r][3] = fmaf(pk, gv.w, dv[r][3]);
-              dk[r][0] = fmaf(sk, qv.x, dk[r][0]); dk[r][1] = fmaf(sk, qv.y, dk[r][1]);
-              dk[r][2] = fmaf(sk, qv.z, dk[r][2]); dk[r][3] = fmaf(sk, qv.w, dk[r][3]);
+            for (int n = 0; n < NCW; ++n) {
+              const float4 gv = reinterpret_cast<const float4 *>(Gs + (4 * q4 + kk) * RS)[col(n)];
+              const float4 qv = reinterpret_cast<const float4 *>(Qs + (4 * q4 + kk) * RS)[col(n)];
+#pragma unroll
+              for (int r = 0; r < 4; ++r) {
+                const float pk = kk == 0 ? p[r].x : kk == 1 ? p[r].y : kk == 2 ? p[r].z : p[r].w;
+                const float sk = kk == 0 ? s[r].x : kk == 1 ? s[r].y : kk == 2 ? s[r].z : s[r].w;
+                dv[n][r][0] = fmaf(pk, gv.x, dv[n][r][0]); dv[n][r][1] = fmaf(pk, gv.y, dv[n][r][1]);
+                dv[n][r][2] = fmaf(pk, gv.z, dv[n][r][2]); dv[n][r][3] = fmaf(pk, gv.w, dv[n][r][3]);
+                dk[n][r][0] = fmaf(sk, qv.x, dk[n][r][0]); dk[n][r][1] = fmaf(sk, qv.y, dk[n][r][1]);
+                dk[n][r][2] = fmaf(sk, qv.z, dk[n][r][2]); dk[n][r][3] = fmaf(sk, qv.w, dk[n][r][3]);
+              }
             }
           }
         }
@@ -451,12 +481,16 @@ __global__ void __launch_bounds__(BB_THREADS, 2)
   }
   if (out_thread) {
 #pragma unroll
-    for (int r = 0; r < 4; ++r) {
-      const int kj = k0 + rg * 4 + r;
-      if (kj >= Sq) continue;
-      float *base = dqkv + (row0 + kj) * ld + head * hd;
-      reinterpret_cast<float4 *>(base + d)[cg] = make_float4(dk[r][0], dk[r][1], dk[r][2], dk[r][3]);
-      reinterpret_cast<float4 *>(base + 2 * d)[cg] = make_float4(dv[r][0], dv[r][1], dv[r][2], dv[r][3]);
+    for (int n = 0; n < NCW; ++n) {
+      if (!col_ok(n)) continue;
+#pragma unroll
+      for (int r = 0; r < 4; ++r) {
+        const int kj = k0 + rg * 4 + r;
+        if (kj >= Sq) continue;
+        float *base = dqkv + (row0 + kj) * ld + head * hd;
+        reinterpret_cast<float4 *>(base + d)[col(n)] = make_float4(dk[n][r][0], dk[n][r][1], dk[n][r][2], dk[n][r][3]);
+        reinterpret_cast<float4 *>(base + 2 * d)[col(n)] = make_float4(dv[n][r][0], dv[n][r][1], dv[n][r][2], dv[n][r][3]);
+      }
     }
   }
 }
@@ -521,7 +555,7 @@ extern "C" int mts_embed_bwd(const float *dpre, int B, int S, int d, float *dpos
   return 0;
 }
 
-template <bool DROP>
+template <bool DROP, int NCW>
 static int band_attn_bwd_launch(const float *qkv, int64_t ld, const float *o, const float *d_o, const float *lse,
                                 const int32_t *lengths, const int32_t *offsets, int B, int S, int nheads, int hd, int w,
                                 float *dqkv, float *delta_ws, float p_drop, uint64_t seed, void *stream) {
@@ -531,20 +565,20 @@ static int band_attn_bwd_launch(const float *qkv, int64_t ld, const float *o, co
   MTS_PER_DEVICE(size_t, set_dq);   // one pair per instantiation and device
   MTS_PER_DEVICE(size_t, set_dkv);
   if (smem_dq > set_dq) {
-    MTS_CUDA(cudaFuncSetAttribute(band_attn_bwd_dq_kernel<DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_dq));
+    MTS_CUDA(cudaFuncSetAttribute(band_attn_bwd_dq_kernel<DROP, NCW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_dq));
     set_dq = smem_dq;
   }
   if (smem_dkv > set_dkv) {
-    MTS_CUDA(cudaFuncSetAttribute(band_attn_bwd_dkv_kernel<DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_dkv));
+    MTS_CUDA(cudaFuncSetAttribute(band_attn_bwd_dkv_kernel<DROP, NCW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_dkv));
     set_dkv = smem_dkv;
   }
   cudaStream_t st = (cudaStream_t)stream;
   const dim3 grid((S + BB_OWN - 1) / BB_OWN, nheads, B);
   const uint32_t p24 = DROP ? attn_drop_p24(p_drop) : 0u;
   const float inv_keep = DROP ? 1.0f / (1.0f - p_drop) : 1.0f;
-  band_attn_bwd_dq_kernel<DROP><<<grid, BB_THREADS, smem_dq, st>>>(qkv, ld, o, d_o, lse, lengths, offsets, S, nheads, hd, w,
+  band_attn_bwd_dq_kernel<DROP, NCW><<<grid, BB_THREADS, smem_dq, st>>>(qkv, ld, o, d_o, lse, lengths, offsets, S, nheads, hd, w,
                                                                    dqkv, delta_ws, p24, inv_keep, seed);
-  band_attn_bwd_dkv_kernel<DROP><<<grid, BB_THREADS, smem_dkv, st>>>(qkv, ld, d_o, lse, delta_ws, lengths, offsets, S, nheads,
+  band_attn_bwd_dkv_kernel<DROP, NCW><<<grid, BB_THREADS, smem_dkv, st>>>(qkv, ld, d_o, lse, delta_ws, lengths, offsets, S, nheads,
                                                                      hd, w, dqkv, p24, inv_keep, seed);
   MTS_LAUNCH_CHECK();
   return 0;
@@ -555,13 +589,18 @@ extern "C" int mts_band_attn_bwd_dropout(const float *qkv, int64_t ld, const flo
                                          int w, float *dqkv, float *delta_ws, float p_drop, uint64_t seed, void *stream) {
   MTS_REQUIRE(qkv && o && d_o && lse && lengths && dqkv && delta_ws, MTS_E_BADARG, "band_attn_bwd: null pointer");
   MTS_REQUIRE(B > 0 && S > 0 && nheads > 0 && hd > 0 && w >= 0, MTS_E_BADARG, "band_attn_bwd: bad shape");
-  MTS_REQUIRE(hd % 4 == 0 && hd <= 128, MTS_E_UNSUPPORTED, "band_attn_bwd: head dim must be a multiple of 4 and <= 128");
+  MTS_REQUIRE(hd % 4 == 0 && hd <= 256, MTS_E_UNSUPPORTED, "band_attn_bwd: head dim must be a multiple of 4 and <= 256");
   MTS_REQUIRE(ld % 4 == 0 && ld >= 3 * nheads * hd, MTS_E_BADARG, "band_attn_bwd: qkv row stride");
   MTS_REQUIRE(p_drop >= 0.0f && p_drop < 1.0f, MTS_E_BADARG, "band_attn_bwd: dropout probability must be in [0, 1)");
   MTS_REQUIRE(p_drop == 0.0f || S <= (1 << 20), MTS_E_UNSUPPORTED, "band_attn_bwd: dropout indices need S <= 2^20");
+  if (hd > 128) {
+    if (p_drop > 0.0f)
+      return band_attn_bwd_launch<true, 2>(qkv, ld, o, d_o, lse, lengths, offsets, B, S, nheads, hd, w, dqkv, delta_ws, p_drop, seed, stream);
+    return band_attn_bwd_launch<false, 2>(qkv, ld, o, d_o, lse, lengths, offsets, B, S, nheads, hd, w, dqkv, delta_ws, 0.0f, 0ull, stream);
+  }
   if (p_drop > 0.0f)
-    return band_attn_bwd_launch<true>(qkv, ld, o, d_o, lse, lengths, offsets, B, S, nheads, hd, w, dqkv, delta_ws, p_drop, seed, stream);
-  return band_attn_bwd_launch<false>(qkv, ld, o, d_o, lse, lengths, offsets, B, S, nheads, hd, w, dqkv, delta_ws, 0.0f, 0ull, stream);
+    return band_attn_bwd_launch<true, 1>(qkv, ld, o, d_o, lse, lengths, offsets, B, S, nheads, hd, w, dqkv, delta_ws, p_drop, seed, stream);
+  return band_attn_bwd_launch<false, 1>(qkv, ld, o, d_o, lse, lengths, offsets, B, S, nheads, hd, w, dqkv, delta_ws, 0.0f, 0ull, stream);
 }
 
 extern "C" int mts_band_attn_bwd(const float *qkv, int64_t ld, const float *o, const float *d_o, const float *lse,

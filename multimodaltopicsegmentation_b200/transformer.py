@@ -369,9 +369,9 @@ def encoder_forward_f16(x, lens, packed: PackedEncoder, nheads, reaches):
 
 def _bf16_eligible(d, nheads):
     """The bf16 encoder (ops.set_precision("bf16")) serves widths that are whole 32-column blocks (the packed operands carry no K
-    padding) and the head dims of the tcgen05 attention kernels; everything else keeps the fp32 path."""
+    padding) and the head dims of the bf16 attention kernel; everything else keeps the fp32 path."""
     return (ops.PRECISION == "bf16" and _pad32(d) == d and d <= 2048
-            and ops._lib.load().mts_band_attn_tc_supported(d // nheads) != 0)
+            and ops._lib.load().mts_band_attn_bf16_supported(d // nheads) != 0)
 
 
 def encoder_forward_bf16(x, lens, packed: PackedEncoder, nheads, reaches):
