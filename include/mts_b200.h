@@ -353,6 +353,23 @@ int mts_embed_ln_fwd_f16(const float *x, int64_t x_bstride, const float *pos, co
                          const int32_t *lengths, const int32_t *offsets, void *stream);
 int mts_add_ln_fwd_f16(const float *a, const float *res, const float *gamma, const float *beta, int M, int d, float eps, float *y,
                        void *pieces, int K64, float *row_scale, void *stream);
+/* The embeddings LayerNorms over an early-fusion PAIR read in place: x[b, t, :] = [src1[b, t, :D1] | src2[b, t, :D2]], each
+ * source [B, S, D_i] with dense rows (row pitch D_i) and its own batch stride bstride_i (elements), d = D1 + D2.  Every output,
+ * and every other argument, as in mts_embed_ln_fwd / mts_embed_ln_fwd_f16 / mts_embed_ln_fwd_bf16in for the concatenated
+ * tensor, bit for bit.  D1 % 4 == 0, D2 % 4 == 0; sources on 16 bytes (fp32) or 8 bytes (bf16), bstride_i % 4 == 0; otherwise
+ * MTS_E_UNSUPPORTED (concatenate and call the single-source entry). */
+int mts_embed_ln_fwd_pair(const float *src1, int64_t bstride1, int D1, const float *src2, int64_t bstride2, int D2,
+                          const float *pos, const float *typ, const float *gamma, const float *beta, int B, int S, float eps,
+                          float *y, float *y_hi, float *y_lo, int Kp, float *sum_out, float *stats, const int32_t *lengths,
+                          const int32_t *offsets, void *stream);
+int mts_embed_ln_fwd_f16_pair(const float *src1, int64_t bstride1, int D1, const float *src2, int64_t bstride2, int D2,
+                              const float *pos, const float *typ, const float *gamma, const float *beta, int B, int S, float eps,
+                              float *y, void *pieces, int K64, float *row_scale, const int32_t *lengths, const int32_t *offsets,
+                              void *stream);
+int mts_embed_ln_fwd_bf16in_pair(const void *src1, int64_t bstride1, int D1, const void *src2, int64_t bstride2, int D2,
+                                 const float *pos, const float *typ, const float *gamma, const float *beta, int B, int S,
+                                 float eps, float *y, float *y_lo, int Kp, const int32_t *lengths, const int32_t *offsets,
+                                 void *stream);
 /* LongformerIntermediate (:1103-1116) activation fused with the operand split: hi/lo [rows,Kp] of GELU(src);
  * act [rows,cols] or NULL: GELU(src) in fp32, kept for the weight gradient of the next dense layer. */
 int mts_gelu_split(const float *src, int64_t ld, int rows, int cols, int Kp, float *act, float *hi, float *lo,

@@ -68,6 +68,12 @@ SIGNATURES = {
                                  _P]),
     "mts_embed_ln_fwd_f16": (c_int, [_P, c_int64, _P, _P, _P, _P, c_int, c_int, c_int, c_float, _P, _P, c_int, _P, _P, _P, _P]),
     "mts_add_ln_fwd_f16": (c_int, [_P, _P, _P, _P, c_int, c_int, c_float, _P, _P, c_int, _P, _P]),
+    "mts_embed_ln_fwd_pair": (c_int, [_P, c_int64, c_int, _P, c_int64, c_int, _P, _P, _P, _P, c_int, c_int, c_float, _P, _P, _P, c_int,
+                                      _P, _P, _P, _P, _P]),
+    "mts_embed_ln_fwd_f16_pair": (c_int, [_P, c_int64, c_int, _P, c_int64, c_int, _P, _P, _P, _P, c_int, c_int, c_float, _P, _P, c_int,
+                                          _P, _P, _P, _P]),
+    "mts_embed_ln_fwd_bf16in_pair": (c_int, [_P, c_int64, c_int, _P, c_int64, c_int, _P, _P, _P, _P, c_int, c_int, c_float, _P, _P,
+                                             c_int, _P, _P, _P]),
     "mts_add_ln_fwd": (c_int, [_P, _P, _P, _P, c_int, c_int, c_float, _P, _P, _P, c_int, _P, _P, _P]),
     "mts_gelu_split": (c_int, [_P, c_int64, c_int, c_int, c_int, _P, _P, _P, _P]),
     "mts_band_attn_fwd": (c_int, [_P, c_int64, _P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, c_int, _P, _P]),

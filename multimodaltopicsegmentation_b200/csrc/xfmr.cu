@@ -33,7 +33,10 @@ constexpr int LN_MAXV = 16;  // float4 per lane -> d <= 2048 (MAXV = 8 serves d 
 // PIECES: instead of the (hi, lo) pair the kernel writes the fp16-split operand of mts_gemm_f16x3 -- y_lo then points to
 // __half pieces [M][2][Kp] (Kp a multiple of 64: fp16 elements) and row_scale [M] receives 2^-s, where 2^s is the exact
 // power of two that puts the row's largest |y| into [2^13, 2^14) (a warp owns a row, so its maximum is one shuffle tree away).
-template <int MODE, int MAXV, bool PIECES = false>
+// PAIR (MODE 0 / 2): x is the early-fusion concatenation [a | a2] read in place -- float4 columns below d1 / 4 come from
+// a[b, t, :d1], the rest from a2[b, t, :d - d1] (batch stride a2_bstride); everything from the sum on is unchanged, so the
+// outputs equal those for the concatenated tensor bit for bit.
+template <int MODE, int MAXV, bool PIECES = false, bool PAIR = false>
 __global__ void __launch_bounds__(256) ln_fwd_kernel(const float *__restrict__ a, int64_t a_bstride,
                                                      const float *__restrict__ b, const float *__restrict__ typ,
                                                      const float *__restrict__ gamma, const float *__restrict__ beta,
@@ -41,12 +44,15 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const float *__restrict__ a
                                                      float *__restrict__ y_hi, float *__restrict__ y_lo, int Kp,
                                                      float *__restrict__ sum_out, float *__restrict__ stats,
                                                      const int32_t *__restrict__ lengths,
-                                                     const int32_t *__restrict__ offsets, float *__restrict__ row_scale = nullptr) {
+                                                     const int32_t *__restrict__ offsets, float *__restrict__ row_scale = nullptr,
+                                                     const float *__restrict__ a2 = nullptr, int64_t a2_bstride = 0, int d1 = 0) {
+  static_assert(!PAIR || MODE != 1, "a second source is an embeddings-LayerNorm form");
   const int lane = threadIdx.x & 31;
   const int nv = d >> 2;
+  const int nv1 = PAIR ? d1 >> 2 : nv;
   const int warps = (gridDim.x * blockDim.x) >> 5;
   for (int in_row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; in_row < M; in_row += warps) {
-    const float4 *pa, *pb;
+    const float4 *pa, *pb, *pa2 = nullptr;
     int row = in_row;
     if (MODE != 1) {
       const int bi = in_row / S, t = in_row % S;
@@ -54,10 +60,18 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const float *__restrict__ a
         if (t >= lengths[bi]) continue;
         row = offsets[bi] + t;
       }
+      const int w1 = PAIR ? d1 : d;   // row pitch of the (first) source
       if (MODE == 2)   // 4 bf16 (8 bytes) per float4 column: pa is only a row address here, read as uint2 below
-        pa = reinterpret_cast<const float4 *>(reinterpret_cast<const uint16_t *>(a) + (int64_t)bi * a_bstride + (int64_t)t * d);
+        pa = reinterpret_cast<const float4 *>(reinterpret_cast<const uint16_t *>(a) + (int64_t)bi * a_bstride + (int64_t)t * w1);
       else
-        pa = reinterpret_cast<const float4 *>(a + (int64_t)bi * a_bstride + (int64_t)t * d);
+        pa = reinterpret_cast<const float4 *>(a + (int64_t)bi * a_bstride + (int64_t)t * w1);
+      if (PAIR) {   // row address of the second source, less the d1 / 4 columns of the first: column c reads pa2[c]
+        if (MODE == 2)
+          pa2 = reinterpret_cast<const float4 *>(reinterpret_cast<const uint16_t *>(a2) + (int64_t)bi * a2_bstride +
+                                                 (int64_t)t * (d - d1) - d1);
+        else
+          pa2 = reinterpret_cast<const float4 *>(a2 + (int64_t)bi * a2_bstride + (int64_t)t * (d - d1) - d1);
+      }
       pb = reinterpret_cast<const float4 *>(b + (int64_t)(t + 2) * d);
     } else {
       pa = reinterpret_cast<const float4 *>(a + (int64_t)row * d);
@@ -67,6 +81,20 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const float *__restrict__ a
     // correction operand goes out in 16-byte pieces (corr_store8)
 #define LN_COL(i) (2 * (lane + 32 * ((i) >> 1)) + ((i) & 1))
     float4 v[MAXV];
+    uint2 u2[PAIR && MODE == 2 ? MAXV : 1];
+    if (PAIR) {
+      // every column's load first: with the per-column source select in the loop below, the compiler branches per column
+      // and each load would wait for the previous column's sums
+#pragma unroll
+      for (int i = 0; i < MAXV; ++i) {
+        const int c = LN_COL(i);
+        if (c < nv) {
+          const float4 *src = c >= nv1 ? pa2 : pa;
+          if (MODE == 2) u2[i] = __ldg(reinterpret_cast<const uint2 *>(src) + c);
+          else v[i] = __ldg(src + c);
+        }
+      }
+    }
     float s = 0.0f;
 #pragma unroll
     for (int i = 0; i < MAXV; ++i) {
@@ -74,11 +102,11 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const float *__restrict__ a
       if (c < nv) {
         float4 x;
         if (MODE == 2) {
-          const uint2 u = __ldg(reinterpret_cast<const uint2 *>(pa) + c);
+          const uint2 u = PAIR ? u2[PAIR ? i : 0] : __ldg(reinterpret_cast<const uint2 *>(pa) + c);
           x = make_float4(__uint_as_float(u.x << 16), __uint_as_float(u.x & 0xFFFF0000u), __uint_as_float(u.y << 16),
                           __uint_as_float(u.y & 0xFFFF0000u));
         } else {
-          x = __ldg(pa + c);
+          x = PAIR ? v[i] : __ldg(pa + c);
         }
         if (MODE != 1 || pb) {
           const float4 r = __ldg(pb + c);
@@ -816,6 +844,93 @@ extern "C" int mts_add_ln_fwd_f16(const float *a, const float *res, const float 
   ln_fwd_kernel<1, 8, true><<<grid, 256, 0, (cudaStream_t)stream>>>(a, 0, res, nullptr, gamma, beta, M, 0, d, eps, y, nullptr,
                                                                      reinterpret_cast<float *>(pieces), K64, nullptr, nullptr, nullptr,
                                                                      nullptr, row_scale);
+  MTS_LAUNCH_CHECK();
+  return 0;
+}
+
+// The three embeddings LayerNorms over an early-fusion pair read in place (ln_fwd_kernel<..., PAIR = true>).  `align` is the
+// byte alignment of one float4 column's load: 16 for fp32 sources, 8 for bf16 ones.
+static int ln_pair_ok(const void *src1, int64_t bstride1, int D1, const void *src2, int64_t bstride2, int D2, int align) {
+  if (!src1 || !src2) { set_error("embed_ln_fwd pair: null source"); return MTS_E_BADARG; }
+  if (D1 <= 0 || D2 <= 0) { set_error("embed_ln_fwd pair: empty source width"); return MTS_E_BADARG; }
+  if (D1 % 4 != 0 || D2 % 4 != 0) { set_error("embed_ln_fwd pair: source widths must be multiples of 4"); return MTS_E_UNSUPPORTED; }
+  if ((((uintptr_t)src1 | (uintptr_t)src2) & (uintptr_t)(align - 1)) != 0 || bstride1 % 4 != 0 || bstride2 % 4 != 0) {
+    set_error("embed_ln_fwd pair: sources must be aligned to their load width, batch strides multiples of 4");
+    return MTS_E_UNSUPPORTED;
+  }
+  return 0;
+}
+
+extern "C" int mts_embed_ln_fwd_pair(const float *src1, int64_t bstride1, int D1, const float *src2, int64_t bstride2, int D2,
+                                     const float *pos, const float *typ, const float *gamma, const float *beta, int B, int S,
+                                     float eps, float *y, float *y_hi, float *y_lo, int Kp, float *sum_out, float *stats,
+                                     const int32_t *lengths, const int32_t *offsets, void *stream) {
+  MTS_REQUIRE(pos && typ && gamma && beta && y, MTS_E_BADARG, "embed_ln_fwd_pair: null pointer");
+  MTS_REQUIRE(!offsets || lengths, MTS_E_BADARG, "embed_ln_fwd_pair: ragged output needs the lengths");
+  MTS_REQUIRE(B > 0 && S > 0, MTS_E_BADARG, "embed_ln_fwd_pair: empty shape");
+  int rc = ln_pair_ok(src1, bstride1, D1, src2, bstride2, D2, 16);
+  if (rc) return rc;
+  const int d = D1 + D2;
+  rc = ln_args_ok("embed_ln_fwd_pair", B * S, d, y_hi, y_lo, Kp);
+  if (rc) return rc;
+  const int M = B * S;
+  const unsigned grid = (unsigned)min((int64_t)(M + 7) / 8, (int64_t)kNumSMs * 8);
+  if (d <= 1024)
+    ln_fwd_kernel<0, 8, false, true><<<grid, 256, 0, (cudaStream_t)stream>>>(src1, bstride1, pos, typ, gamma, beta, M, S, d, eps, y,
+                                                                              y_hi, y_lo, Kp, sum_out, stats, lengths, offsets,
+                                                                              nullptr, src2, bstride2, D1);
+  else
+    ln_fwd_kernel<0, 16, false, true><<<grid, 256, 0, (cudaStream_t)stream>>>(src1, bstride1, pos, typ, gamma, beta, M, S, d, eps, y,
+                                                                               y_hi, y_lo, Kp, sum_out, stats, lengths, offsets,
+                                                                               nullptr, src2, bstride2, D1);
+  MTS_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int mts_embed_ln_fwd_f16_pair(const float *src1, int64_t bstride1, int D1, const float *src2, int64_t bstride2, int D2,
+                                         const float *pos, const float *typ, const float *gamma, const float *beta, int B, int S,
+                                         float eps, float *y, void *pieces, int K64, float *row_scale, const int32_t *lengths,
+                                         const int32_t *offsets, void *stream) {
+  MTS_REQUIRE(pos && typ && gamma && beta && y && pieces && row_scale, MTS_E_BADARG, "embed_ln_fwd_f16_pair: null pointer");
+  MTS_REQUIRE(!offsets || lengths, MTS_E_BADARG, "embed_ln_fwd_f16_pair: ragged output needs the lengths");
+  MTS_REQUIRE(B > 0 && S > 0, MTS_E_BADARG, "embed_ln_fwd_f16_pair: empty shape");
+  int rc = ln_pair_ok(src1, bstride1, D1, src2, bstride2, D2, 16);
+  if (rc) return rc;
+  const int d = D1 + D2;
+  MTS_REQUIRE(d <= 1024, MTS_E_UNSUPPORTED, "embed_ln_fwd_f16_pair: width must be <= 1024");
+  MTS_REQUIRE(K64 % 64 == 0 && K64 >= d, MTS_E_BADARG, "embed_ln_fwd_f16_pair: K64 must be a multiple of 64 and >= d");
+  const int M = B * S;
+  const unsigned grid = (unsigned)min((int64_t)(M + 7) / 8, (int64_t)kNumSMs * 8);
+  ln_fwd_kernel<0, 8, true, true><<<grid, 256, 0, (cudaStream_t)stream>>>(src1, bstride1, pos, typ, gamma, beta, M, S, d, eps, y,
+                                                                           nullptr, reinterpret_cast<float *>(pieces), K64, nullptr,
+                                                                           nullptr, lengths, offsets, row_scale, src2, bstride2, D1);
+  MTS_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int mts_embed_ln_fwd_bf16in_pair(const void *src1, int64_t bstride1, int D1, const void *src2, int64_t bstride2, int D2,
+                                            const float *pos, const float *typ, const float *gamma, const float *beta, int B, int S,
+                                            float eps, float *y, float *y_lo, int Kp, const int32_t *lengths,
+                                            const int32_t *offsets, void *stream) {
+  MTS_REQUIRE(pos && typ && gamma && beta && y, MTS_E_BADARG, "embed_ln_fwd_bf16in_pair: null pointer");
+  MTS_REQUIRE(!offsets || lengths, MTS_E_BADARG, "embed_ln_fwd_bf16in_pair: ragged output needs the lengths");
+  MTS_REQUIRE(B > 0 && S > 0, MTS_E_BADARG, "embed_ln_fwd_bf16in_pair: empty shape");
+  int rc = ln_pair_ok(src1, bstride1, D1, src2, bstride2, D2, 8);
+  if (rc) return rc;
+  const int d = D1 + D2;
+  rc = ln_args_ok("embed_ln_fwd_bf16in_pair", B * S, d, nullptr, y_lo, Kp);
+  if (rc) return rc;
+  const int M = B * S;
+  const float *x1 = reinterpret_cast<const float *>(src1), *x2 = reinterpret_cast<const float *>(src2);
+  const unsigned grid = (unsigned)min((int64_t)(M + 7) / 8, (int64_t)kNumSMs * 8);
+  if (d <= 1024)
+    ln_fwd_kernel<2, 8, false, true><<<grid, 256, 0, (cudaStream_t)stream>>>(x1, bstride1, pos, typ, gamma, beta, M, S, d, eps, y,
+                                                                              nullptr, y_lo, Kp, nullptr, nullptr, lengths, offsets,
+                                                                              nullptr, x2, bstride2, D1);
+  else
+    ln_fwd_kernel<2, 16, false, true><<<grid, 256, 0, (cudaStream_t)stream>>>(x1, bstride1, pos, typ, gamma, beta, M, S, d, eps, y,
+                                                                               nullptr, y_lo, Kp, nullptr, nullptr, lengths, offsets,
+                                                                               nullptr, x2, bstride2, D1);
   MTS_LAUNCH_CHECK();
   return 0;
 }

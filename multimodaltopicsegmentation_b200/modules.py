@@ -26,8 +26,11 @@ IMPOSSIBLE = -1e4  # models/CRF.py:95
 
 
 def _lens(lengths, x):
+    """Lengths of a batch whose embeddings x are a [B, T, D] tensor or an early-fusion pair of them (time axis of the first)."""
     if isinstance(lengths, ops.Lengths):
         return lengths
+    if isinstance(x, (tuple, list)):
+        x = x[0]
     return ops.Lengths(lengths, x.device, x.shape[1])
 
 

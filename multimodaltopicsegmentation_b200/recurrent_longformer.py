@@ -253,6 +253,8 @@ class RecurrentLongformer(nn.Module):
         _build_head(self, out_dim, tagset_size, loss_fn, threshold, alpha, gamma)
 
     def _features(self, x, lens):
+        """x: [B, S, embedding_dim] or an early-fusion pair (text, audio); only the first block's RNN reads the pair (in its input
+        projection), later blocks get the previous block's output."""
         for block in self.model:
             x = block(x, lens)
         return x

@@ -22,7 +22,7 @@ import torch
 import torch.nn as nn
 
 from . import ops
-from .modules import _build_head, _head_decode, _head_decode_device, _head_loss
+from .modules import _build_head, _head_decode, _head_decode_device, _head_loss, _lens
 
 _ptr, _call, _stream, _pad32 = ops._ptr, ops._call, ops._stream, ops._pad32
 
@@ -201,9 +201,18 @@ class PackedEncoder:
         return ent
 
 
-def _ln(mode, a, b, typ, gamma, beta, B, S, d, want_split, save, lens=None):
-    """mode 0: embeddings LN over x=a [B,S,d] with position table b (lens given: ragged output rows);
-    mode 1: LN(a + b) over [M,d] rows (M = B, S = 1)."""
+def _split_src(x):
+    """Encoder input -> (x1, x2, B, S, d): x is [B,S,d] embeddings (x2 None) or an early-fusion pair (x1 [B,S,D1], x2 [B,S,D2]),
+    which the embeddings LayerNorm reads in place as [x1 | x2], d = D1 + D2."""
+    if isinstance(x, tuple):
+        x1, x2 = x
+        return x1, x2, x1.shape[0], x1.shape[1], x1.shape[2] + x2.shape[2]
+    return (x, None, *x.shape)
+
+
+def _ln(mode, a, b, typ, gamma, beta, B, S, d, want_split, save, lens=None, a2=None):
+    """mode 0: embeddings LN over x=a [B,S,d] with position table b (lens given: ragged output rows), or over x = [a | a2]
+    when the second source a2 is given; mode 1: LN(a + b) over [M,d] rows (M = B, S = 1)."""
     M = lens.N if lens is not None else B * S
     dev = a.device
     y = torch.empty((M, d), device=dev, dtype=torch.float32)
@@ -214,7 +223,11 @@ def _ln(mode, a, b, typ, gamma, beta, B, S, d, want_split, save, lens=None):
         hi = None if kp == d else torch.empty((M, kp), device=dev, dtype=torch.float32)
     pre = torch.empty((M, d), device=dev, dtype=torch.float32) if save else None
     stats = torch.empty((M, 2), device=dev, dtype=torch.float32) if save else None
-    if mode == 0:
+    if mode == 0 and a2 is not None:
+        _call("mts_embed_ln_fwd_pair", _ptr(a), a.stride(0), a.shape[2], _ptr(a2), a2.stride(0), a2.shape[2], _ptr(b), _ptr(typ),
+              _ptr(gamma), _ptr(beta), B, S, LN_EPS, _ptr(y), _ptr(hi), _ptr(lo), kp, _ptr(pre), _ptr(stats),
+              _ptr(lens.dev) if lens is not None else 0, _ptr(lens.offs) if lens is not None else 0, _stream())
+    elif mode == 0:
         _call("mts_embed_ln_fwd", _ptr(a), a.stride(0), _ptr(b), _ptr(typ), _ptr(gamma), _ptr(beta), B, S, d, LN_EPS,
               _ptr(y), _ptr(hi), _ptr(lo), kp, _ptr(pre), _ptr(stats), _ptr(lens.dev) if lens is not None else 0,
               _ptr(lens.offs) if lens is not None else 0, _stream())
@@ -224,7 +237,7 @@ def _ln(mode, a, b, typ, gamma, beta, B, S, d, want_split, save, lens=None):
     return y, (y if (want_split and hi is None) else hi), lo, pre, stats
 
 
-def _ln_f16(mode, a, b, typ, gamma, beta, B, S, d, lens=None):
+def _ln_f16(mode, a, b, typ, gamma, beta, B, S, d, lens=None, a2=None):
     """_ln for inference with the fp16-split operand of mts_gemm_f16x3 as the second output: (y, pieces [M, 2, K64], scale [M])."""
     M = lens.N if lens is not None else B * S
     dev = a.device
@@ -232,7 +245,11 @@ def _ln_f16(mode, a, b, typ, gamma, beta, B, S, d, lens=None):
     y = torch.empty((M, d), device=dev, dtype=torch.float32)
     pieces = torch.empty((M, 2, k64), device=dev, dtype=torch.float16)
     scale = torch.empty((M,), device=dev, dtype=torch.float32)
-    if mode == 0:
+    if mode == 0 and a2 is not None:
+        _call("mts_embed_ln_fwd_f16_pair", _ptr(a), a.stride(0), a.shape[2], _ptr(a2), a2.stride(0), a2.shape[2], _ptr(b), _ptr(typ),
+              _ptr(gamma), _ptr(beta), B, S, LN_EPS, _ptr(y), _ptr(pieces), k64, _ptr(scale), _ptr(lens.dev) if lens is not None else 0,
+              _ptr(lens.offs) if lens is not None else 0, _stream())
+    elif mode == 0:
         _call("mts_embed_ln_fwd_f16", _ptr(a), a.stride(0), _ptr(b), _ptr(typ), _ptr(gamma), _ptr(beta), B, S, d, LN_EPS, _ptr(y),
               _ptr(pieces), k64, _ptr(scale), _ptr(lens.dev) if lens is not None else 0, _ptr(lens.offs) if lens is not None else 0,
               _stream())
@@ -315,7 +332,7 @@ def encoder_forward_f16(x, lens, packed: PackedEncoder, nheads, reaches):
                -> intermediate dense + GELU [f16x3 when F >= 256, writes (z, z_lo)] -> output dense [tf32x3] -> LN(u + y) -> ...
 
     Same arithmetic contract as encoder_forward (fp32-grade products: relative error ~2^-22 instead of ~2^-19)."""
-    B, S, d = x.shape
+    x, x2, B, S, d = _split_src(x)
     ragged = LAYOUT == "ragged"
     M = lens.N if ragged else B * S
     offs = _ptr(lens.offs) if ragged else 0
@@ -324,7 +341,7 @@ def encoder_forward_f16(x, lens, packed: PackedEncoder, nheads, reaches):
     m = packed.params
     emb = m.embeddings
     h, h_p, h_s = _ln_f16(0, x, emb.position_embeddings.weight.detach(), emb.token_type_embeddings.weight.detach()[0],
-                          emb.LayerNorm.weight.detach(), emb.LayerNorm.bias.detach(), B, S, d, lens if ragged else None)
+                          emb.LayerNorm.weight.detach(), emb.LayerNorm.bias.detach(), B, S, d, lens if ragged else None, a2=x2)
     n_layers = len(m.encoder.layer)
     for l in range(n_layers):
         lyr = m.encoder.layer[l]
@@ -383,8 +400,8 @@ def encoder_forward_bf16(x, lens, packed: PackedEncoder, nheads, reaches):
                -> intermediate dense + GELU [bf16p_gelu_pair: z, z_lo] -> output dense [bf16p] -> LN(u + y) -> ...
 
     The residual stream, the LayerNorm statistics, the softmax, all accumulators and the returned hidden state are fp32.
-    x may be fp32 or bfloat16 embeddings (read as they are: half the bytes)."""
-    B, S, d = x.shape
+    x may be fp32 or bfloat16 embeddings (read as they are: half the bytes), or an early-fusion pair of either."""
+    x, x2, B, S, d = _split_src(x)
     ragged = LAYOUT == "ragged"
     M = lens.N if ragged else B * S
     offs = _ptr(lens.offs) if ragged else 0
@@ -396,12 +413,17 @@ def encoder_forward_bf16(x, lens, packed: PackedEncoder, nheads, reaches):
     if x.dtype == torch.bfloat16:
         h = torch.empty((M, d), device=dev, dtype=torch.float32)
         h_lo = torch.empty((M, d), device=dev, dtype=torch.float32)
-        _call("mts_embed_ln_fwd_bf16in", _ptr(x), x.stride(0), _ptr(pos), _ptr(typ), _ptr(emb.LayerNorm.weight.detach()),
-              _ptr(emb.LayerNorm.bias.detach()), B, S, d, LN_EPS, _ptr(h), _ptr(h_lo), d, _ptr(lens.dev) if ragged else 0, offs,
-              _stream())
+        if x2 is not None:
+            _call("mts_embed_ln_fwd_bf16in_pair", _ptr(x), x.stride(0), x.shape[2], _ptr(x2), x2.stride(0), x2.shape[2], _ptr(pos),
+                  _ptr(typ), _ptr(emb.LayerNorm.weight.detach()), _ptr(emb.LayerNorm.bias.detach()), B, S, LN_EPS, _ptr(h), _ptr(h_lo),
+                  d, _ptr(lens.dev) if ragged else 0, offs, _stream())
+        else:
+            _call("mts_embed_ln_fwd_bf16in", _ptr(x), x.stride(0), _ptr(pos), _ptr(typ), _ptr(emb.LayerNorm.weight.detach()),
+                  _ptr(emb.LayerNorm.bias.detach()), B, S, d, LN_EPS, _ptr(h), _ptr(h_lo), d, _ptr(lens.dev) if ragged else 0, offs,
+                  _stream())
     else:
         h, _, h_lo, _, _ = _ln(0, x, pos, typ, emb.LayerNorm.weight.detach(), emb.LayerNorm.bias.detach(), B, S, d, True, False,
-                               lens if ragged else None)
+                               lens if ragged else None, a2=x2)
     n_layers = len(m.encoder.layer)
     for l in range(n_layers):
         lyr = m.encoder.layer[l]
@@ -442,14 +464,16 @@ def encoder_forward(x, lens, packed: PackedEncoder, nheads, reaches, save, p_hid
     p_hidden > 0 applies HF's `hidden_dropout_prob` at its three sites (after the embeddings LayerNorm and on the
     two dense outputs that feed a residual LayerNorm: modeling_longformer.py LongformerEmbeddings / SelfOutput /
     Output) as plain element-wise passes -- a training-time regulariser, not part of the timed inference path.
-    p_attn > 0 applies HF's `attention_probs_dropout_prob` inside the attention kernel (one seed per layer)."""
-    B, S, d = x.shape
+    p_attn > 0 applies HF's `attention_probs_dropout_prob` inside the attention kernel (one seed per layer).
+    x may also be an early-fusion pair (x1 [B,S,D1], x2 [B,S,D2]) of the sources the embeddings LayerNorm reads in place."""
+    _, _, B, S, d = _split_src(x)
     ragged = LAYOUT == "ragged"
     M = lens.N if ragged else B * S
     if not save and p_hidden == 0 and p_attn == 0 and _bf16_eligible(d, nheads):
         return encoder_forward_bf16(x, lens, packed, nheads, reaches), None
     if not save and p_hidden == 0 and p_attn == 0 and not FOLD_RESIDUAL and _f16x3_eligible(M, d, 0, ops):
         return encoder_forward_f16(x, lens, packed, nheads, reaches), None
+    x, x2 = _split_src(x)[:2]
     offs = _ptr(lens.offs) if ragged else 0
     dev = x.device
     hd = d // nheads
@@ -458,7 +482,7 @@ def encoder_forward(x, lens, packed: PackedEncoder, nheads, reaches, save, p_hid
     emb = m.embeddings
     h, h_hi, h_lo, pre0, st0 = _ln(0, x, emb.position_embeddings.weight.detach(), emb.token_type_embeddings.weight.detach()[0],
                                    emb.LayerNorm.weight.detach(), emb.LayerNorm.bias.detach(), B, S, d, True, save,
-                                   lens if ragged else None)
+                                   lens if ragged else None, a2=x2)
     masks = []
     if p_hidden > 0:
         h = _drop(h, 0, p_hidden, masks)
@@ -531,8 +555,20 @@ def encoder_forward(x, lens, packed: PackedEncoder, nheads, reaches, save, p_hid
     return h.view(B, S, d), saved
 
 
+def _encoder_input(parts):
+    """[x] -> x; [x1, x2] -> the pair (x1, x2) when the embeddings LayerNorm can read it in place (widths multiples of 4, sources
+    aligned to the load width: 16 bytes for fp32, 8 for bf16, batch strides multiples of 4), else its concatenation on the
+    device (same values: the single-source path)."""
+    if len(parts) == 1:
+        return parts[0]
+    align = 16 if parts[0].dtype == torch.float32 else 8
+    if all(t.shape[2] % 4 == 0 and t.data_ptr() % align == 0 and t.stride(0) % 4 == 0 for t in parts):
+        return tuple(parts)
+    return torch.cat(parts, dim=-1)
+
+
 class EncoderFn(torch.autograd.Function):
-    """Differentiable w.r.t. the encoder parameters (the input embeddings are data)."""
+    """Differentiable w.r.t. the encoder parameters (the input embeddings, a tensor or an early-fusion pair, are data)."""
 
     @staticmethod
     def forward(ctx, x, lens, packed, nheads, reaches, p_hidden, p_attn, *params):
@@ -540,7 +576,7 @@ class EncoderFn(torch.autograd.Function):
         out, saved = encoder_forward(x, lens, packed, nheads, reaches, save=need, p_hidden=p_hidden, p_attn=p_attn)
         if need:
             ctx.saved, ctx.lens, ctx.packed, ctx.nheads, ctx.reaches = saved, lens, packed, nheads, reaches
-            ctx.shape = x.shape
+            ctx.shape = _split_src(x)[2:]
         return out
 
     @staticmethod
@@ -577,31 +613,47 @@ class Longformer_Local_Attention(nn.Module):
         return self._packed
 
     def forward(self, src, lengths):
-        if torch.is_tensor(src) and src.dtype == torch.bfloat16:   # bf16 embeddings: inference under ops.set_precision("bf16")
-            x = ops._check(src, "src", torch.bfloat16)
+        """src: [B, S, d_model] embeddings, or an early-fusion pair (text [B, S, D1], audio [B, S, D2]) with D1 + D2 = d_model,
+        which the embeddings LayerNorm reads in place instead of their concatenation (same results, bit for bit)."""
+        pair = isinstance(src, (tuple, list))
+        if pair:
+            if len(src) != 2 or not all(torch.is_tensor(t) for t in src):
+                raise TypeError("src: an early-fusion input is a pair (text, audio) of [B, S, D_i] tensors")
+            if src[0].dtype != src[1].dtype:
+                raise TypeError(f"src: both members of the pair must have one dtype, got {src[0].dtype} and {src[1].dtype}")
+        parts = list(src) if pair else [src]
+        if torch.is_tensor(parts[0]) and parts[0].dtype == torch.bfloat16:   # bf16 embeddings: inference under ops.set_precision("bf16")
+            parts = [ops._check(t, "src", torch.bfloat16) for t in parts]
             if ops.PRECISION != "bf16":
                 raise TypeError("src: bfloat16 embeddings belong to the bf16 path (ops.set_precision('bf16')); the fp32 path takes fp32")
         else:
-            x = ops._check(src, "src")
-        if x.dim() != 3 or x.shape[2] != self.d_model:
+            parts = [ops._check(t, "src") for t in parts]
+        x = parts[0]
+        if pair:
+            x2 = parts[1]
+            if x.dim() != 3 or x2.dim() != 3 or x.shape[:2] != x2.shape[:2] or x.shape[2] + x2.shape[2] != self.d_model:
+                raise ValueError(f"expected a pair of [B, S, D_i] embeddings with D1 + D2 = {self.d_model}, got {tuple(x.shape)} "
+                                 f"and {tuple(x2.shape)}")
+        elif x.dim() != 3 or x.shape[2] != self.d_model:
             raise ValueError(f"expected [B, S, {self.d_model}] embeddings, got {tuple(x.shape)}")
         if x.shape[1] + 2 > self.max_positions:
             raise IndexError(f"sequence length {x.shape[1]} exceeds the position table ({self.max_positions} rows, "
                              "position ids start at 2)")
         p_hidden = self.hidden_dropout if self.training else 0.0
         p_attn = self.attention_dropout if self.training else 0.0   # HF attention_probs_dropout_prob (RestrictedTransformerLayer.py:92)
-        if x.stride(2) != 1 or x.stride(1) != x.shape[2]:
-            x = x.contiguous()
+        parts = [t if (t.stride(2) == 1 and t.stride(1) == t.shape[2]) else t.contiguous() for t in parts]
         lens = lengths if isinstance(lengths, ops.Lengths) else ops.Lengths(lengths, x.device, x.shape[1])
         packed = self.packed()
         params = packed.used_parameters()
         if not (torch.is_grad_enabled() and any(p.requires_grad for p in params)):  # inference: nothing saved
             if x.dtype == torch.bfloat16 and not (p_hidden == 0 and p_attn == 0 and _bf16_eligible(self.d_model, self.nhead)):
-                x = x.float()   # a shape or dropout setting the bf16 encoder does not serve: the fp32 path, on the same values
-            return encoder_forward(x, lens, packed, self.nhead, self.reaches, save=False, p_hidden=p_hidden, p_attn=p_attn)[0]
+                # a shape or dropout setting the bf16 encoder does not serve: the fp32 path, on the same values
+                parts = [t.float() for t in parts]
+            return encoder_forward(_encoder_input(parts), lens, packed, self.nhead, self.reaches, save=False, p_hidden=p_hidden,
+                                   p_attn=p_attn)[0]
         if x.dtype == torch.bfloat16:
             raise NotImplementedError("bfloat16 embeddings serve inference only (ops.set_precision('bf16')): train in fp32")
-        return EncoderFn.apply(x, lens, packed, self.nhead, self.reaches, p_hidden, p_attn, *params)
+        return EncoderFn.apply(_encoder_input(parts), lens, packed, self.nhead, self.reaches, p_hidden, p_attn, *params)
 
 
 class Transformer_segmenter(nn.Module):
@@ -620,18 +672,19 @@ class Transformer_segmenter(nn.Module):
                                                 tagset_size=tagset_size, device=None, max_position_embedding=4096)
         _build_head(self, embedding_dim, tagset_size, loss_fn, threshold, alpha, gamma)
 
+    # xs: [B, S, embedding_dim] embeddings or an early-fusion pair (text, audio) of [B, S, D_i] (Longformer_Local_Attention.forward)
     def loss(self, xs, lengths, tags, segments=None, global_count=None):
         if segments is not None:
             raise NotImplementedError("the auxiliary cosine loss (segments=...) is outside the B200 hot path")
-        lens = ops.Lengths(lengths, xs.device, xs.shape[1]) if not isinstance(lengths, ops.Lengths) else lengths
+        lens = _lens(lengths, xs)
         return _head_loss(self, self.model(xs, lens), lens, tags, global_count)
 
     def forward(self, xs, lenghts, threshold=0.4):
-        lens = ops.Lengths(lenghts, xs.device, xs.shape[1]) if not isinstance(lenghts, ops.Lengths) else lenghts
+        lens = _lens(lenghts, xs)
         with torch.no_grad():
             return _head_decode(self, self.model(xs, lens), lens, threshold)
 
     def decode_device(self, xs, lenghts, threshold=0.4):
-        lens = ops.Lengths(lenghts, xs.device, xs.shape[1]) if not isinstance(lenghts, ops.Lengths) else lenghts
+        lens = _lens(lenghts, xs)
         with torch.no_grad():
             return (*_head_decode_device(self, self.model(xs, lens), lens, threshold), lens)
